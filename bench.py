@@ -7,7 +7,7 @@ the same state u_s every time: u_s is the PNP solution converged on refinement l
 flow: PB Newton -> interpolate(BCExtension) -> PNP Newton) and carried to the fine mesh by P1 interpolation
 (nested iteration), i.e. a late Newton step of a production run.  value = dofs / step time.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--levels L] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--levels L] [--impl reference] [--dump-outputs DIR]
 
 N > 1 (torchrun, one rank per GPU): the SAME global problem is split into N subdomains (strong scaling); NCCL carries
 halo values and scalar sums only (DESIGN.md "multi-GPU").
@@ -312,6 +312,25 @@ def parity_vs_n1(args, c, capi, u_vec, fine, rank, world, dist, torch, cfg, a, j
     return val
 
 
+DUMP_VERTICES = 1 << 21   # --dump-outputs: at most this many vertices of u (3 x 8 B each, 48 MiB)
+
+
+def dump_outputs(path, u, r):
+    """--dump-outputs: what a caller of the timed step receives from its last call, so that two builds can be compared output
+    for output.  u.npy: the updated state as (3, nv) float64 (phi, c+, c- in mesh vertex order); on meshes with more than
+    DUMP_VERTICES vertices, the columns of a fixed seeded sample of vertices (sorted, the same on every run).
+    newton_result.npy: converged, iterations, first defect, defect, reduction, linear iterations, line-search trials,
+    Jacobian assemblies, residual assemblies (float64)."""
+    os.makedirs(path, exist_ok=True)
+    u = np.asarray(u, dtype=np.float64).reshape(3, -1)
+    if u.shape[1] > DUMP_VERTICES:
+        u = u[:, np.sort(np.random.default_rng(0).choice(u.shape[1], DUMP_VERTICES, replace=False))]
+    np.save(os.path.join(path, "u.npy"), np.ascontiguousarray(u))
+    np.save(os.path.join(path, "newton_result.npy"), np.array(
+        [r.converged, r.iterations, r.first_defect, r.defect, r.reduction, r.linear_iterations, r.line_search_trials,
+         r.jacobian_assemblies, r.residual_assemblies], dtype=np.float64))
+
+
 def run_gpu(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -384,6 +403,8 @@ def run_gpu(args, rank, world, local_rank):
     n_spmv, spmv_ms = c.profile_spmv_get()
     c.profile_spmv(False)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:   # before the end-to-end leg below overwrites u
+        dump_outputs(args.dump_outputs, c.download(u, 3), stats[-1])
     # ---- end-to-end: same step through the C ABI with host buffers (H2D of u, D2H of the updated u) ----
     step(True)
     barrier()
@@ -510,7 +531,13 @@ def main():
     ap.add_argument("--replica-level", type=int, default=3, help="N > 1: levels below this one run replicated on every rank (no halo exchanges there)")
     ap.add_argument("--python-partitioner", action="store_true", help="N > 1: numpy partitioner (dune_pnp_b200/partition.py) instead of the native one")
     ap.add_argument("--dense-coarse", action="store_true", help="N > 1: replicated dense LU on the Gmsh mesh instead of the replica hierarchy")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's outputs to DIR/*.npy "
+                    "(one GPU, b200 implementation)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs the b200 implementation on one GPU")
     global DENSE_COARSE, REPLICA_LEVEL, PYTHON_PARTITIONER
     DENSE_COARSE = args.dense_coarse; REPLICA_LEVEL = args.replica_level; PYTHON_PARTITIONER = args.python_partitioner
     for kv in args.solver_opt:

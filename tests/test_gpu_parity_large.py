@@ -98,6 +98,27 @@ def test_pore_golden_solution():
     assert abs(r2.first_defect - d[0]) <= 1e-10 * d[0]
 
 
+def test_bench_dump_outputs_are_reproducible(tmp_path):
+    """`bench.py --dump-outputs` at k = 4 (2.2 M dofs): the last timed Newton step's state and result are written, and a
+    second run with the same arguments writes the same bits (the start state and the step are deterministic), so that two
+    builds can be compared output for output."""
+    import json
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    lines = {}
+    for run in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--levels", "4", "--steps", "2", "--warmup", "1",
+                              "--no-cpu", "--dump-outputs", str(tmp_path / run)], capture_output=True, text=True, timeout=900)
+        assert out.returncode == 0, out.stderr[-3000:]
+        lines[run] = json.loads(out.stdout.strip().splitlines()[-1])
+    u, res = np.load(tmp_path / "a" / "u.npy"), np.load(tmp_path / "a" / "newton_result.npy")
+    assert u.dtype == np.float64 and u.shape == (3, 738033) and np.all(np.isfinite(u))
+    assert res.dtype == np.float64 and res[1] == 1 and res[3] == lines["a"]["defect_after"] and res[3] < res[2]
+    for name in ("u.npy", "newton_result.npy"):
+        assert np.array_equal(np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name)), name
+
+
 def _smooth_state(m, op):
     """A smooth, physically shaped state (potential O(1), concentrations around c0) plus deterministic noise."""
     rng = np.random.RandomState(21)

@@ -205,6 +205,29 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_bench_dump_outputs_writes_a_fixed_sample_within_64_mb(tmp_path):
+    """`bench.py --dump-outputs`: a small state is written whole; a larger one as the same seeded, sorted vertex sample on
+    every call (all three fields of each sampled vertex), float64, at most 64 MB in all."""
+    import bench
+    from dune_pnp_b200 import capi
+    r = capi.NewtonResult()
+    r.converged, r.iterations, r.first_defect, r.defect, r.linear_iterations = 0, 1, 3.4, 1.5e-5, 5
+    small = np.arange(3 * 1000, dtype=np.float64)
+    bench.dump_outputs(str(tmp_path / "s"), small, r)
+    assert np.array_equal(np.load(tmp_path / "s" / "u.npy"), small.reshape(3, -1))
+    res = np.load(tmp_path / "s" / "newton_result.npy")
+    assert res.dtype == np.float64 and list(res[:4]) == [0, 1, 3.4, 1.5e-5] and res[5] == 5
+    nv = bench.DUMP_VERTICES + 12345
+    big = np.arange(3 * nv, dtype=np.float64)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), big, r)
+    a, b = np.load(tmp_path / "a" / "u.npy"), np.load(tmp_path / "b" / "u.npy")
+    assert a.dtype == np.float64 and a.shape == (3, bench.DUMP_VERTICES) and np.array_equal(a, b)
+    idx = a[0].astype(np.int64)
+    assert np.all(np.diff(idx) > 0) and np.array_equal(a[1], idx + nv) and np.array_equal(a[2], idx + 2 * nv)
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 64e6
+
+
 def test_shared_sinh_is_bit_identical_on_both_sides_and_accurate():
     """SURVEY H1: the PB source term's sinh is one sequence of +, -, *, /, floor on the device (pnp_elem.cuh: pnp_sinh,
     compiled here for the host without FMA contraction) and in the oracle (sinh_shared): same bits, within 4 ulp of libm."""

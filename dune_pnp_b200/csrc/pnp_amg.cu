@@ -10,7 +10,8 @@
 // iteration counts therefore differ from ISTL's; Newton counts do not (SURVEY H3).
 //
 // Point-block hierarchy: all fields of a vertex are aggregated together, so every level keeps the
-// 1-plane (scalar) or 7-plane (PNP) layout of the fine matrix and runs the same SpMV.
+// 1-plane (scalar), 7-plane or compact 5-plane (PNP) layout of the fine matrix and runs the same SpMV.  The Galerkin sums
+// are linear in the planes, so a compact level's coarse operator is the compact form of the 7-plane one.
 // Symbolic phase (aggregates, coarse patterns, gather lists) once per mesh/operator type;
 // numeric phase (Galerkin sums, inverse diagonals) per Jacobian -- deterministic gathers, no atomics.
 #include <cub/cub.cuh>
@@ -239,6 +240,7 @@ __global__ void k_galerkin(const int* __restrict__ seg_ptr, const int* __restric
           const unsigned m = dmask[wv];
           if (m && rpf[wv] == s[q]) {
             if (NP == 1) { if ((m >> comp0) & 1u) v[q][0] = 0.0; }
+            else if (NP == PNP_COMPACT_PLANES) { if (m & 1u) v[q][0] = 0.0; } // all three fields: L = 1, D = 0
             else {
               if (m & 1u) v[q][0] = 0.0;
               if (m & 2u) v[q][NP == 7 ? 4 : 0] = 0.0;
@@ -269,8 +271,8 @@ __global__ void k_dinv(const int* __restrict__ rp, const double* __restrict__ va
     if (NP == 1) { const double d = vals[s]; dinv[v] = d != 0.0 ? 1.0 / d : 0.0; }
     else {
       // B = [a b c; d e 0; f 0 g]
-      const double a = vals[s], b = vals[stride + s], c_ = vals[2 * stride + s], d = vals[3 * stride + s],
-                   e = vals[4 * stride + s], f = vals[5 * stride + s], g = vals[6 * stride + s];
+      const PnpBlock B = pnp_block_at<NP>(vals, stride, s);
+      const double a = B.a, b = B.b, c_ = B.c, d = B.d, e = B.e, f = B.f, g = B.g;
       const double det = a * e * g - b * d * g - c_ * e * f;
       double* o = dinv + 9l * v;
       const double scale = fabs(a * e * g) + fabs(b * d * g) + fabs(c_ * e * f);
@@ -320,11 +322,13 @@ __global__ void k_gershgorin(const int* __restrict__ rp, const double* __restric
     } else {
       double s0_ = 0.0, s1_ = 0.0, s2_ = 0.0;
       for (int s = s0; s < s1; s++) {
-        s0_ += fabs(vals[s]) + fabs(vals[stride + s]) + fabs(vals[2 * stride + s]);
-        s1_ += fabs(vals[3 * stride + s]) + fabs(vals[4 * stride + s]);
-        s2_ += fabs(vals[5 * stride + s]) + fabs(vals[6 * stride + s]);
+        const PnpBlock B = pnp_block_at<NP>(vals, stride, s);
+        s0_ += fabs(B.a) + fabs(B.b) + fabs(B.c);
+        s1_ += fabs(B.d) + fabs(B.e);
+        s2_ += fabs(B.f) + fabs(B.g);
       }
-      const double d0 = fabs(vals[s0]), d1 = fabs(vals[4 * stride + s0]), d2 = fabs(vals[6 * stride + s0]);
+      const PnpBlock D = pnp_block_at<NP>(vals, stride, s0);
+      const double d0 = fabs(D.a), d1 = fabs(D.e), d2 = fabs(D.g);
       if (d0 > 0.0) best = fmax(best, s0_ / d0);
       if (d1 > 0.0) best = fmax(best, s1_ / d1);
       if (d2 > 0.0) best = fmax(best, s2_ / d2);
@@ -426,13 +430,12 @@ __global__ void k_dense_fill_global(const int* __restrict__ rp, const unsigned* 
       const unsigned dm = (dmask && s == rp[r]) ? dmask[r] : 0u;
       if (NP == 1) { if (!((dm >> comp0) & 1u)) atomicAdd(&Ad[cg * n + rg], vals[s]); }
       else {
+        const PnpBlock B = pnp_block_at<NP>(vals, stride, s);
 #pragma unroll
         for (int ki = 0; ki < 3; ki++)
 #pragma unroll
-          for (int kj = 0; kj < 3; kj++) {
-            const int pl = pnp_plane(ki, kj);
-            if (pl >= 0 && !(ki == kj && ((dm >> ki) & 1u))) atomicAdd(&Ad[(F * cg + kj) * n + F * rg + ki], vals[pl * stride + s]);
-          }
+          for (int kj = 0; kj < 3; kj++)
+            if (pnp_plane(ki, kj) >= 0 && !(ki == kj && ((dm >> ki) & 1u))) atomicAdd(&Ad[(F * cg + kj) * n + F * rg + ki], B.at(ki, kj));
       }
     }
   }
@@ -501,7 +504,7 @@ template <int EPI>
 void level_op(Ctx& c, const Amg& A, const Level& l, const double* x, const double* b, double* y, double omega_or_c2 = -1.0,
               double c1 = 0.0, double* dvec = nullptr) {
   StarOpArgs a{l.rp, l.col, l.vals, l.nslots, l.nv, x, y};
-  a.b = b; a.dinv = l.dinv.p; a.block = A.NP == 7; a.omega = omega_or_c2 < 0 ? A.omega : omega_or_c2; a.c1 = c1; a.dvec = dvec;
+  a.b = b; a.dinv = l.dinv.p; a.block = A.F == 3; a.omega = omega_or_c2 < 0 ? A.omega : omega_or_c2; a.c1 = c1; a.dvec = dvec;
   const bool fine = &l == A.L[0].get();
   if (A.distributed) halo_exchange(*l.lc, const_cast<double*>(x), A.F); // ghost columns of the iterate
   if (fine) c.prof_mark(EPI == EPI_RESIDUAL ? 1 : 2);
@@ -649,7 +652,7 @@ void coarsen_geometric(Ctx& c, Amg& A, int li, const HierLevel& h, const int* in
 
 void alloc_work(Ctx& c, Amg& A, Level& l) {
   const size_t n = (size_t)A.F * l.nv, nall = (A.distributed && l.lc) ? (size_t)A.F * l.lc->nv : n;
-  l.dinv.alloc(A.NP == 7 ? 9 * (size_t)l.nv : n); l.x.alloc(nall); l.x2.alloc(nall); l.b.alloc(nall); l.r.alloc(nall);
+  l.dinv.alloc(A.F == 3 ? 9 * (size_t)l.nv : n); l.x.alloc(nall); l.x2.alloc(nall); l.b.alloc(nall); l.r.alloc(nall);
   l.x.zero(c.stream); l.x2.zero(c.stream); l.b.zero(c.stream); l.r.zero(c.stream);
 }
 
@@ -681,7 +684,7 @@ void coarsen_distributed(Ctx& c, Amg& A, int li, MgLevelRef& ref) {
   nl->lc = &kc; nl->nv = nvc; nl->nslots = kc.nslots; nl->rp = kc.rp.p; nl->col = kc.adj.p;
   nl->dm = kc.dmask.p;
   nl->u.fields = A.F; nl->u.d.alloc((size_t)A.F * kc.nv); nl->u.d.zero(c.stream);
-  nl->Amat.op = A.NP == 7 ? OP_PNP : OP_PB; nl->Amat.nplanes = A.NP;
+  nl->Amat.op = A.F == 3 ? OP_PNP : OP_PB; nl->Amat.nplanes = A.NP;
   nl->Amat.vals.alloc((size_t)A.NP * kc.nslots);
   nl->vals = nl->Amat.vals.p;
   A.L.push_back(std::move(nl));
@@ -703,16 +706,25 @@ const double* level_values(Ctx& c, Amg& A, int li, const double* uf, int comp0) 
     c.acct(Ctx::ACC_TRANSFER, 8.0 * l.nv + 16.0 * A.F * n.nv);
     Operator op = c.last_op; op.aux0 = op.aux1 = -1;
     assemble_jacobian_on(c, StarView{n.rp, n.col, n.xy_own.p, n.dmask_own.p, n.nv}, n.nslots, op, n.u.d.p, n.vals_own.p,
-                         c.last_mode, c.last_eps);
+                         A.NP, c.last_mode, c.last_eps);
     return n.u.d.p;
   }
   // constrained dofs of the finer level are left out of the product (only their unit diagonal has to be skipped)
   if (A.NP == 1)
     KL(c, k_galerkin<1>, n.nslots, l.seg_ptr.p, l.seg_items.p, l.seg_w.p, n.nslots, l.vals, l.nslots, n.vals_own.p, l.dm, l.col, l.rp, comp0);
+  else if (A.NP == PNP_COMPACT_PLANES)
+    KL(c, k_galerkin<PNP_COMPACT_PLANES>, n.nslots, l.seg_ptr.p, l.seg_items.p, l.seg_w.p, n.nslots, l.vals, l.nslots, n.vals_own.p, l.dm, l.col, l.rp, comp0);
   else
     KL(c, k_galerkin<7>, n.nslots, l.seg_ptr.p, l.seg_items.p, l.seg_w.p, n.nslots, l.vals, l.nslots, n.vals_own.p, l.dm, l.col, l.rp, comp0);
   c.acct(Ctx::ACC_ASSEMBLY, 8.0 * A.NP * ((double)l.nslots + (double)n.nslots) + 5.0 * (double)l.seg_items.n + 4.0 * (double)n.nslots);
   return nullptr;
+}
+
+// smoother matrix of level l (k_dinv)
+void level_dinv(Ctx& c, Amg& A, Level& l) {
+  if (A.NP == 1) KL(c, k_dinv<1>, l.nv, l.rp, l.vals, l.nslots, l.nv, l.dinv.p);
+  else if (A.NP == PNP_COMPACT_PLANES) KL(c, k_dinv<PNP_COMPACT_PLANES>, l.nv, l.rp, l.vals, l.nslots, l.nv, l.dinv.p);
+  else KL(c, k_dinv<7>, l.nv, l.rp, l.vals, l.nslots, l.nv, l.dinv.p);
 }
 
 // Gershgorin bounds of D^-1 A on every level (Chebyshev smoother); distributed: the maximum over the ranks
@@ -722,6 +734,7 @@ void gershgorin_bounds(Ctx& c, Amg& A) {
   for (size_t li = 0; li < A.L.size(); li++) {
     Level& l = *A.L[li];
     if (A.NP == 1) KL(c, k_gershgorin<1>, l.nv, l.rp, l.vals, l.nslots, l.nv, d_l.p + li);
+    else if (A.NP == PNP_COMPACT_PLANES) KL(c, k_gershgorin<PNP_COMPACT_PLANES>, l.nv, l.rp, l.vals, l.nslots, l.nv, d_l.p + li);
     else KL(c, k_gershgorin<7>, l.nv, l.rp, l.vals, l.nslots, l.nv, d_l.p + li);
   }
   if (A.distributed) allreduce_max_u64(c, d_l.p, A.L.size());
@@ -754,9 +767,8 @@ void numeric(Ctx& c, Amg& A, int comp0) {
     }
     for (size_t li = 0; li < A.L.size(); li++) {
       Level& l = *A.L[li];
-      if (A.NP == 1) KL(c, k_dinv<1>, l.nv, l.rp, l.vals, l.nslots, l.nv, l.dinv.p);
-      else KL(c, k_dinv<7>, l.nv, l.rp, l.vals, l.nslots, l.nv, l.dinv.p);
-      c.acct(Ctx::ACC_ASSEMBLY, (4.0 + 8.0 * A.NP + (A.NP == 7 ? 72.0 : 8.0)) * l.nv);
+      level_dinv(c, A, l);
+      c.acct(Ctx::ACC_ASSEMBLY, (4.0 + 8.0 * A.NP + (A.F == 3 ? 72.0 : 8.0)) * l.nv);
     }
     if (c.mg_replica) replica_setup(c, A); else dense_factor_global(c, A);
     if (A.smoother == 1) gershgorin_bounds(c, A);
@@ -766,9 +778,8 @@ void numeric(Ctx& c, Amg& A, int comp0) {
   for (size_t li = 0; li < A.L.size(); li++) {
     Level& l = *A.L[li];
     if (li + 1 < A.L.size()) uf = level_values(c, A, (int)li, uf, comp0);
-    if (A.NP == 1) KL(c, k_dinv<1>, l.nv, l.rp, l.vals, l.nslots, l.nv, l.dinv.p);
-    else KL(c, k_dinv<7>, l.nv, l.rp, l.vals, l.nslots, l.nv, l.dinv.p);
-    c.acct(Ctx::ACC_ASSEMBLY, (4.0 + 8.0 * A.NP + (A.NP == 7 ? 72.0 : 8.0)) * l.nv);
+    level_dinv(c, A, l);
+    c.acct(Ctx::ACC_ASSEMBLY, (4.0 + 8.0 * A.NP + (A.F == 3 ? 72.0 : 8.0)) * l.nv);
   }
   A.dense_n = 0;
   if ((long)A.F * A.L.back()->nv <= A.dense_max) dense_factor(c, A); // (a one-level hierarchy is a direct solve)
@@ -786,13 +797,12 @@ __global__ void k_dense_fill(const int* __restrict__ rp, const unsigned* __restr
       if (cidx >= nv) continue;
       if (NP == 1) Ad[cidx * n + r] = vals[s];
       else {
+        const PnpBlock B = pnp_block_at<NP>(vals, stride, s);
 #pragma unroll
         for (int ki = 0; ki < 3; ki++)
 #pragma unroll
-          for (int kj = 0; kj < 3; kj++) {
-            const int pl = pnp_plane(ki, kj);
-            if (pl >= 0) Ad[(F * cidx + kj) * n + F * r + ki] = vals[pl * stride + s];
-          }
+          for (int kj = 0; kj < 3; kj++)
+            if (pnp_plane(ki, kj) >= 0) Ad[(F * cidx + kj) * n + F * r + ki] = B.at(ki, kj);
       }
     }
 }
@@ -813,6 +823,7 @@ void dense_factor(Ctx& c, Amg& A) {
   if (A.dense.n != (size_t)(n * n)) { A.dense.alloc(n * n); A.dense_piv.alloc(n); A.dense_info.alloc(1); }
   A.dense.zero(c.stream);
   if (A.NP == 1) KL(c, k_dense_fill<1>, l.nv, l.rp, l.col, l.vals, l.nslots, l.nv, A.dense.p, n);
+  else if (A.NP == PNP_COMPACT_PLANES) KL(c, k_dense_fill<PNP_COMPACT_PLANES>, l.nv, l.rp, l.col, l.vals, l.nslots, l.nv, A.dense.p, n);
   else KL(c, k_dense_fill<7>, l.nv, l.rp, l.col, l.vals, l.nslots, l.nv, A.dense.p, n);
   KL(c, k_dense_fix_diag, n, A.dense.p, n);
   int lwork = 0;
@@ -843,6 +854,8 @@ void dense_factor_global(Ctx& c, Amg& A) {
   A.dense.zero(c.stream);
   const unsigned char* dm = c.mg_aggregated ? l.lc->dmask.p : nullptr;
   if (A.NP == 1) KL(c, k_dense_fill_global<1>, l.nv, l.rp, l.col, l.vals, l.nslots, l.nv, c.mg_gid.p, A.dense.p, n, dm, A.comp0);
+  else if (A.NP == PNP_COMPACT_PLANES)
+    KL(c, k_dense_fill_global<PNP_COMPACT_PLANES>, l.nv, l.rp, l.col, l.vals, l.nslots, l.nv, c.mg_gid.p, A.dense.p, n, dm, A.comp0);
   else KL(c, k_dense_fill_global<7>, l.nv, l.rp, l.col, l.vals, l.nslots, l.nv, c.mg_gid.p, A.dense.p, n, dm, A.comp0);
   allreduce_sum(c, A.dense.p, (size_t)(n * n));
   KL(c, k_dense_fix_diag, n, A.dense.p, n);
@@ -935,7 +948,7 @@ void replica_solve(Ctx& c, Amg& A, Level& l, int nu) {
 void jacobi0(Ctx& c, Amg& A, Level& l, double omega, double* dvec) {
   if (A.F == 1) KL(c, k_jacobi0<1>, l.nv, l.dinv.p, l.b.p, omega, l.x.p, l.nv, dvec);
   else KL(c, k_jacobi0<3>, l.nv, l.dinv.p, l.b.p, omega, l.x.p, l.nv, dvec);
-  c.acct(Ctx::ACC_TRANSFER, ((A.NP == 7 ? 72.0 : 8.0) + 16.0 * A.F + (dvec ? 8.0 * A.F : 0.0)) * l.nv);
+  c.acct(Ctx::ACC_TRANSFER, ((A.F == 3 ? 72.0 : 8.0) + 16.0 * A.F + (dvec ? 8.0 * A.F : 0.0)) * l.nv);
 }
 
 // `steps` smoothing steps on level l for A x = b; zero: x starts from 0.  Result in l.x.
@@ -1155,6 +1168,7 @@ void amg_setup(Ctx& c, Solver& S, const Matrix& M) {
   A.coarse_sweeps = (int)S.opt("amg_coarse_sweeps", 40); A.smoother = (int)S.opt("amg_smoother", 0);
   PNP_REQUIRE(A.smoother >= 0 && A.smoother <= 2, PNP_E_ARG, "amg_smoother: 0 damped Jacobi, 1 Chebyshev, 2 symmetric Gauss-Seidel");
   PNP_REQUIRE(A.smoother != 2 || !A.distributed, PNP_E_ARG, "the Gauss-Seidel smoother sweeps the rows of one GPU: use Jacobi / Chebyshev on a partitioned mesh");
+  PNP_REQUIRE(A.smoother != 2 || A.NP != PNP_COMPACT_PLANES, PNP_E_ARG, "the Gauss-Seidel smoother sweeps 7-plane PNP matrices only");
   A.cheb_ratio = S.opt("amg_cheb_ratio", 8.0);
   A.pre_steps = (int)S.opt("amg_pre_steps", -1); A.post_steps = (int)S.opt("amg_post_steps", -1);
   numeric(c, A, comp0);

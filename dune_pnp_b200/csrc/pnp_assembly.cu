@@ -28,11 +28,10 @@ namespace {
 constexpr int JAC_CHUNK = 128;   // = block size
 constexpr int JAC_CAP = 1152;    // staged slots per plane
 
-template <int OP, int MODE>
+template <int OP, int MODE, int NP>
 __global__ void __launch_bounds__(JAC_CHUNK)
 k_jacobian(StarView M, PhysParams P, const double* __restrict__ u, const double* __restrict__ aux0,
            const double* __restrict__ aux1, double eps, int comp0, double* __restrict__ vals, long stride) {
-  constexpr int NP = OpTraits<OP>::NPLANES;
   extern __shared__ double stage[]; // NP * JAC_CAP
   const int nchunks = (M.nv + JAC_CHUNK - 1) / JAC_CHUNK;
   for (int ch = blockIdx.x; ch < nchunks; ch += gridDim.x) {
@@ -40,35 +39,42 @@ k_jacobian(StarView M, PhysParams P, const double* __restrict__ u, const double*
     const int sb = M.rp[v0], n = M.rp[v1] - sb;
     const int v = v0 + threadIdx.x;
     if (n <= JAC_CAP) { // block-uniform
-      if (v < v1) jacobian_row<OP, MODE>(M, P, u, aux0, aux1, eps, comp0, v, stage, JAC_CAP, sb);
+      if (v < v1) jacobian_row<OP, MODE, NP>(M, P, u, aux0, aux1, eps, comp0, v, stage, JAC_CAP, sb);
       __syncthreads();
 #pragma unroll
       for (int p = 0; p < NP; p++)
         for (int i = threadIdx.x; i < n; i += JAC_CHUNK) vals[p * stride + sb + i] = stage[p * JAC_CAP + i];
       __syncthreads();
     } else if (v < v1) {
-      jacobian_row<OP, MODE>(M, P, u, aux0, aux1, eps, comp0, v, vals, stride);
+      jacobian_row<OP, MODE, NP>(M, P, u, aux0, aux1, eps, comp0, v, vals, stride);
     }
   }
 }
 
 // M: the star to assemble on -- the context's own (finest) one, or a coarser refinement level's (multigrid)
-template <int OP, int MODE>
+template <int OP, int MODE, int NP = OpTraits<OP>::NPLANES>
 void launch_jac(Ctx& c, const StarView& M, const Operator& op, const double* u, const double* a0, const double* a1,
                 double* vals, long stride, double eps) {
   const PhysParams P = c.phys(op.valency);
-  const int smem = OpTraits<OP>::NPLANES * JAC_CAP * (int)sizeof(double);
+  const int smem = NP * JAC_CAP * (int)sizeof(double);
   // (set on every launch: the attribute is per device and a process may drive several contexts)
-  PNP_CUDA(cudaFuncSetAttribute(k_jacobian<OP, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  PNP_CUDA(cudaFuncSetAttribute(k_jacobian<OP, MODE, NP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   const int grid = grid_for(M.nv, JAC_CHUNK, c.sm_count * 16);
-  k_jacobian<OP, MODE><<<grid, JAC_CHUNK, smem, c.stream>>>(M, P, u, a0, a1, eps, op.comp0, vals, stride);
+  k_jacobian<OP, MODE, NP><<<grid, JAC_CHUNK, smem, c.stream>>>(M, P, u, a0, a1, eps, op.comp0, vals, stride);
   PNP_CHECK_LAUNCH(); c.launches++;
   // ring (4 B/slot), row pointer + coordinates + Dirichlet mask + state (+ coefficient fields) per vertex, NP planes written
-  c.acct(Ctx::ACC_ASSEMBLY, (4.0 + 8.0 * OpTraits<OP>::NPLANES) * (double)stride + (21.0 + 8.0 * OpTraits<OP>::F + 8.0 * OpTraits<OP>::NAUX) * (double)M.nv);
+  c.acct(Ctx::ACC_ASSEMBLY, (4.0 + 8.0 * NP) * (double)stride + (21.0 + 8.0 * OpTraits<OP>::F + 8.0 * OpTraits<OP>::NAUX) * (double)M.nv);
 }
+// nplanes: the layout of the target matrix (the compact PNP layout is assembled by the exact derivative only)
 template <int MODE>
 void dispatch_jac(Ctx& c, const StarView& M, const Operator& op, const double* u, const double* a0, const double* a1,
-                  double* vals, long stride, double eps) {
+                  double* vals, long stride, double eps, int nplanes) {
+  if constexpr (MODE == JAC_ANALYTIC) {
+    if (op.op == OP_PNP && nplanes == PNP_COMPACT_PLANES) {
+      launch_jac<OP_PNP, JAC_ANALYTIC, PNP_COMPACT_PLANES>(c, M, op, u, a0, a1, vals, stride, eps);
+      return;
+    }
+  }
   switch (op.op) {
     case OP_PB: launch_jac<OP_PB, MODE>(c, M, op, u, a0, a1, vals, stride, eps); break;
     case OP_POISSON: launch_jac<OP_POISSON, MODE>(c, M, op, u, a0, a1, vals, stride, eps); break;
@@ -241,7 +247,7 @@ void launch_jac_fdw(Ctx& c, const StarView& M, const Operator& op, const double*
 
 void launch_jacobian_fd(Ctx& c, const StarView& M, const Operator& op, const double* u, const double* a0, const double* a1,
                         double* vals, long stride, double eps) {
-  if (!tune().fd_warp) { dispatch_jac<JAC_FD_FAITHFUL>(c, M, op, u, a0, a1, vals, stride, eps); return; }
+  if (!tune().fd_warp) { dispatch_jac<JAC_FD_FAITHFUL>(c, M, op, u, a0, a1, vals, stride, eps, op_planes(op.op)); return; }
   switch (op.op) {
     case OP_PB: launch_jac_fdw<OP_PB>(c, M, op, u, a0, a1, vals, stride, eps); break;
     case OP_POISSON: launch_jac_fdw<OP_POISSON>(c, M, op, u, a0, a1, vals, stride, eps); break;
@@ -344,23 +350,27 @@ void assemble_jacobian(Ctx& c, const Operator& op, Vec& u, Matrix& A, int mode, 
   PNP_REQUIRE(u.fields == op_fields(op.op), PNP_E_ARG, "vector field count does not match the operator");
   PNP_REQUIRE(A.op == op.op, PNP_E_ARG, "matrix belongs to another operator type");
   PNP_REQUIRE(mode == JAC_FD_FAITHFUL || mode == JAC_ANALYTIC, PNP_E_ARG, "unknown jacobian mode");
+  PNP_REQUIRE(A.nplanes == op_planes(op.op) || (A.nplanes == PNP_COMPACT_PLANES && op.op == OP_PNP && mode == JAC_ANALYTIC),
+              PNP_E_ARG, "matrix layout does not fit the operator and Jacobian mode");
   const double *a0, *a1;
   coefficient_ptrs(c, op, &a0, &a1);
   A.comp0 = op.comp0;
   c.last_u = u.d.p; c.last_op = op; c.last_mode = mode; c.last_eps = eps; c.last_vals = A.vals.p;
   halo_exchange(c, u.d.p, u.fields);
   if (mode == JAC_FD_FAITHFUL) launch_jacobian_fd(c, c.star(), op, u.d.p, a0, a1, A.vals.p, c.nslots, eps);
-  else dispatch_jac<JAC_ANALYTIC>(c, c.star(), op, u.d.p, a0, a1, A.vals.p, c.nslots, eps);
+  else dispatch_jac<JAC_ANALYTIC>(c, c.star(), op, u.d.p, a0, a1, A.vals.p, c.nslots, eps, A.nplanes);
 }
 
 // The same operator on another star of the same mesh hierarchy (a coarser refinement level held by the multigrid):
-// u in that level's numbering, vals = NPLANES planes of `stride` slots.  Operators with coefficient fields are not
-// supported here (their coefficients live on the finest level only).
-void assemble_jacobian_on(Ctx& c, const StarView& M, long stride, const Operator& op, const double* u, double* vals, int mode,
-                          double eps) {
+// u in that level's numbering, vals = `nplanes` planes of `stride` slots (the layout of the finest level's matrix).
+// Operators with coefficient fields are not supported here (their coefficients live on the finest level only).
+void assemble_jacobian_on(Ctx& c, const StarView& M, long stride, const Operator& op, const double* u, double* vals, int nplanes,
+                          int mode, double eps) {
   PNP_REQUIRE(op.op == OP_PB || op.op == OP_PNP || op.op == OP_MASS, PNP_E_ARG, "no coefficient fields on coarse levels");
+  PNP_REQUIRE(nplanes == op_planes(op.op) || (nplanes == PNP_COMPACT_PLANES && op.op == OP_PNP && mode == JAC_ANALYTIC),
+              PNP_E_ARG, "matrix layout does not fit the operator and Jacobian mode");
   if (mode == JAC_FD_FAITHFUL) launch_jacobian_fd(c, M, op, u, nullptr, nullptr, vals, stride, eps);
-  else dispatch_jac<JAC_ANALYTIC>(c, M, op, u, nullptr, nullptr, vals, stride, eps);
+  else dispatch_jac<JAC_ANALYTIC>(c, M, op, u, nullptr, nullptr, vals, stride, eps, nplanes);
 }
 
 #endif // PNP_ASM_FAITHFUL

@@ -231,6 +231,7 @@ pnp_status pnp_tune(const char* name, double value) {
   else if (n == "tma_lpr") t.tma_lpr = (int)value;
   else if (n == "graph") t.graph = value != 0;
   else if (n == "fd_warp") t.fd_warp = value != 0;
+  else if (n == "jac_compact") t.jac_compact = value != 0;
   else if (n == "p2_chunk") t.p2_chunk = (long)value;
   else if (n == "tma_min_rows") t.tma_min_rows = (long)value;
   else return PNP_E_ARG;

@@ -70,6 +70,7 @@ struct Tune {
   long tma_min_rows = -1; // smallest level the streaming SpMV serves (-1: two tiles per SM)
   int graph = 1;          // the multigrid's coarse correction is replayed from a CUDA graph
   int fd_warp = 1;        // FD-faithful Jacobian: warp-cooperative kernel (0: one thread per vertex)
+  int jac_compact = 1;    // Newton / linear-problem Jacobian in the compact 5-plane PNP layout where it applies (0: always 7)
   long p2_chunk = 0;      // quadratic / cubic elements: elements per scratch block of the Jacobian assembly (0: 2 GB worth)
 };
 inline Tune& tune() { static Tune t; return t; }
@@ -100,7 +101,7 @@ struct Vec {
 };
 struct Matrix {
   int op = 0;
-  int nplanes = 1;
+  int nplanes = 1;   // value planes: 1 (scalar operators), 7 (PNP, pnp_plane()) or 5 (compact PNP, pnp_block())
   int comp0 = 0;  // BC component of the operator that assembled it (scalar operators)
   DBuf<double> vals; // nplanes * nslots (star layout) or csr_nnz (quadratic elements)
   // quadratic elements (pnp_p2.cu): scalar CSR in the reference's dof numbering; the pattern belongs to the space
@@ -312,7 +313,8 @@ void interpolate_bcext(Ctx&, int comp, const Vec* pb, Vec& out);
 // pnp_assembly.cu
 void assemble_residual(Ctx&, const Operator&, Vec& u, Vec& r);   // refreshes the ghost part of u
 void assemble_jacobian(Ctx&, const Operator&, Vec& u, Matrix& A, int mode, double eps);
-void assemble_jacobian_on(Ctx&, const StarView& M, long stride, const Operator&, const double* u, double* vals, int mode, double eps);
+void assemble_jacobian_on(Ctx&, const StarView& M, long stride, const Operator&, const double* u, double* vals, int nplanes,
+                          int mode, double eps);
 // pnp_linalg.cu
 void spmv(Ctx&, const Matrix& A, double* x, double* y); // refreshes the ghost part of x
 double vec_norm(Ctx&, const double* x, long n);

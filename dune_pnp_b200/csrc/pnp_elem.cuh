@@ -49,6 +49,36 @@ PNP_HD constexpr int pnp_plane(int ki, int kj) {
   return ki == 0 ? kj : (ki == 1 ? (kj == 0 ? 3 : (kj == 1 ? 4 : -1)) : (kj == 0 ? 5 : (kj == 2 ? 6 : -1)));
 }
 
+// The exact-derivative PNP Jacobian also comes in a compact layout of 5 planes: the residual has unit coefficients on
+// grad(phi).grad(v), grad(c+).grad(v) and grad(c-).grad(v), so the three diagonal blocks share one Laplacian L, and
+// (phi,c-) is the negation of (phi,c+):
+//   plane 0: L = (phi,phi)    1: M = (phi,c+) = -(phi,c-)    2: (c+,phi)    3: (c-,phi)
+//   plane 4: D, the drift:   (c+,c+) = L - D,  (c-,c-) = L + D
+// It needs every constrained vertex to be constrained in all three fields (one unit diagonal L = 1, D = 0 per vertex).
+// A star SpMV then reads 44 B per slot instead of 60.
+constexpr int PNP_COMPACT_PLANES = 5;
+
+// the 3x3 block [a b c; d e 0; f 0 g] of one slot from its NP value planes (1: scalar a; 5: compact; 7: pnp_plane())
+struct PnpBlock {
+  double a, b, c, d, e, f, g;
+  PNP_HD double at(int ki, int kj) const {
+    return ki == 0 ? (kj == 0 ? a : (kj == 1 ? b : c)) : (ki == 1 ? (kj == 0 ? d : (kj == 1 ? e : 0.0)) : (kj == 0 ? f : (kj == 2 ? g : 0.0)));
+  }
+};
+template <int NP> PNP_HD PnpBlock pnp_block(const double* v) {
+  static_assert(NP == 1 || NP == 5 || NP == 7, "PNP value planes: 1, 5 or 7");
+  if (NP == 1) return PnpBlock{v[0], 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+  if (NP == 5) return PnpBlock{v[0], v[1], -v[1], v[2], v[0] - v[4 % NP], v[3 % NP], v[0] + v[4 % NP]};
+  return PnpBlock{v[0], v[1 % NP], v[2 % NP], v[3 % NP], v[4 % NP], v[5 % NP], v[6 % NP]};
+}
+// ... of slot s of NP planes `stride` doubles apart
+template <int NP> PNP_HD PnpBlock pnp_block_at(const double* vals, long stride, long s) {
+  double v[NP];
+#pragma unroll
+  for (int p = 0; p < NP; p++) v[p] = vals[p * stride + s];
+  return pnp_block<NP>(v);
+}
+
 // Quadrature tables (dune-geometry simplex rules; SURVEY App. A.6): point q of the NQ-point rule.
 template <int NQ> PNP_HD void quad_point(int q, double& xi0, double& xi1, double& w);
 template <> PNP_HD void quad_point<3>(int q, double& xi0, double& xi1, double& w) {
@@ -317,6 +347,45 @@ PNP_HD void jac_rows_exact(const Geo& G, const PhysParams& P, const double (*xl)
         else v = phi[j] * phi[I];
         blk[j][0] += v * factor;
       }
+    }
+  }
+}
+
+// The same exact derivative of the PNP rows in the compact layout (PNP_COMPACT_PLANES).  L, M, (c+,phi) and (c-,phi) are
+// the operations of jac_rows_exact in the same order; D collects the drift terms that planes 4 and 6 add to K there.
+template <int I>
+PNP_HD void jac_rows_exact_compact(const Geo& G, const PhysParams& P, const double (*xl)[3],
+                                   double (*blk)[PNP_COMPACT_PLANES]) {
+  constexpr int NQ = OpTraits<OP_PNP>::NQ;
+  double K[3];
+#pragma unroll
+  for (int j = 0; j < 3; j++) K[j] = G.g[j][0] * G.g[I][0] + G.g[j][1] * G.g[I][1];
+  double gP[2] = {0.0, 0.0};
+#pragma unroll
+  for (int i = 0; i < 3; i++) { gP[0] += xl[0][i] * G.g[i][0]; gP[1] += xl[0][i] * G.g[i][1]; }
+  const double dPI = gP[0] * G.g[I][0] + gP[1] * G.g[I][1];
+#pragma unroll
+  for (int q = 0; q < NQ; q++) {
+    double xi0, xi1, w;
+    quad_point<NQ>(q, xi0, xi1, w);
+    const double phi[3] = {1.0 - xi0 - xi1, xi0, xi1};
+    double factor = w * G.detabs;
+    if (P.cylindrical) {
+      const double gy = G.y0 + (G.y1 - G.y0) * xi0 + (G.y2 - G.y0) * xi1;
+      factor *= gy * 2 * P.PI;
+    }
+    double up = 0.0, um = 0.0;
+#pragma unroll
+    for (int i = 0; i < 3; i++) { up += xl[1][i] * phi[i]; um += xl[2][i] * phi[i]; }
+    const double kap = 4 * P.PI * P.l_b;
+#pragma unroll
+    for (int j = 0; j < 3; j++) {
+      const double m = kap * phi[j] * phi[I] * factor;
+      blk[j][0] += K[j] * factor;
+      blk[j][1] += m;
+      blk[j][2] -= up * K[j] * factor;
+      blk[j][3] += um * K[j] * factor;
+      blk[j][4] += phi[j] * dPI * factor;
     }
   }
 }

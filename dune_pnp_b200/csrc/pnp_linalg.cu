@@ -5,7 +5,7 @@
 // iteration follows dune-istl 2.2 solvers.hh as restated in SURVEY.md App. A.7 (half-iteration
 // counting, convergence tests after each half step, breakdown thresholds 1e-80).
 //
-// All kernels are HBM-bound.  SpMV bytes per launch: NPLANES*8*nslots (values) + 4*nslots (adj)
+// All kernels are HBM-bound.  SpMV bytes per launch: nplanes*8*nslots (values) + 4*nslots (adj)
 // + 4*nv (rp) + 16*F*nv (x read once if the gather hits cache, y written).  Dot products ride in
 // the epilogue of the kernel that produces their operand; reductions are two-stage and
 // deterministic (per-block partials, then one block).
@@ -117,9 +117,10 @@ __global__ void k_diag_inverse(const int* __restrict__ rp, const double* __restr
     const int s = rp[v];
     if (NP == 1) dinv[v] = 1.0 / vals[s];
     else {
-      dinv[(long)F * v] = 1.0 / vals[s];
-      dinv[(long)F * v + 1] = 1.0 / vals[4 * stride + s];
-      dinv[(long)F * v + 2] = 1.0 / vals[6 * stride + s];
+      const PnpBlock B = pnp_block_at<NP>(vals, stride, s);
+      dinv[(long)F * v] = 1.0 / B.a;
+      dinv[(long)F * v + 1] = 1.0 / B.e;
+      dinv[(long)F * v + 2] = 1.0 / B.g;
     }
   }
 }
@@ -219,6 +220,8 @@ void prec_setup(Ctx& c, Solver& S, const Matrix& A) {
     case PNP_PREC_JACOBI: {
       const int g = grid_for(c.n_own, 256);
       if (A.nplanes == 1) k_diag_inverse<1><<<g, 256, 0, c.stream>>>(c.rp.p, A.vals.p, c.nslots, (int)c.n_own, S.dinv.p);
+      else if (A.nplanes == PNP_COMPACT_PLANES)
+        k_diag_inverse<PNP_COMPACT_PLANES><<<g, 256, 0, c.stream>>>(c.rp.p, A.vals.p, c.nslots, (int)c.n_own, S.dinv.p);
       else k_diag_inverse<7><<<g, 256, 0, c.stream>>>(c.rp.p, A.vals.p, c.nslots, (int)c.n_own, S.dinv.p);
       PNP_CHECK_LAUNCH(); c.launches++;
       break;

@@ -14,6 +14,18 @@ namespace pnp {
 
 namespace {
 double now() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+
+// Value planes of the work-space Jacobian: the compact PNP layout (pnp_jacobian_planes) where the solver reads the matrix
+// through star SpMVs and diagonal blocks only -- no preconditioner, Jacobi, or the multigrid with the Jacobi or Chebyshev
+// smoother -- on one GPU.  Everything else keeps the operator's planes.
+int workspace_planes(const Ctx& c, const Operator& op, const Solver& S, int jac_mode) {
+  if (op.op != OP_PNP || !tune().jac_compact || c.n_own != c.nv || !c.mg.empty()) return op_planes(op.op);
+  const double sm = S.opt("amg_smoother", 0);
+  const bool solver_ok = S.prec == PNP_PREC_NONE || S.prec == PNP_PREC_JACOBI || (S.prec == PNP_PREC_AMG && (sm == 0 || sm == 1));
+  std::vector<int> btype;
+  for (const HostSurface& s : c.params.surfaces) btype.insert(btype.end(), s.btype, s.btype + 3);
+  return pnp_jacobian_planes(jac_mode, c.degree, solver_ok, btype.data(), (int)c.params.surfaces.size());
+}
 } // namespace
 
 int newton_apply(Ctx& c, const Operator& op, Vec& u, Solver& S, const pnp_newton_opts& o, pnp_newton_result& R) {
@@ -26,7 +38,7 @@ int newton_apply(Ctx& c, const Operator& op, Vec& u, Solver& S, const pnp_newton
   r.fields = z.fields = prev_u.fields = F;
   if (r.d.n != (size_t)nall) { r.d.alloc(nall); z.d.alloc(nall); prev_u.d.alloc(nall); }
   r.d.zero(c.stream); z.d.zero(c.stream);
-  A.op = op.op; A.nplanes = op_planes(op.op);
+  A.op = op.op; A.nplanes = workspace_planes(c, op, S, o.jac_mode);
   if (c.degree >= 2) p2_matrix_init(c, A, op);
   else if (A.vals.n != (size_t)A.nplanes * c.nslots) A.vals.alloc((size_t)A.nplanes * c.nslots);
   const double t_start = now();
@@ -144,7 +156,7 @@ LinResult slp_apply(Ctx& c, const Operator& op, Vec& u, Solver& S, double reduct
   r.fields = z.fields = F;
   if (r.d.n != (size_t)nall) { r.d.alloc(nall); z.d.alloc(nall); c.ws_prev.d.alloc(nall); }
   r.d.zero(c.stream); z.d.zero(c.stream);
-  A.op = op.op; A.nplanes = op_planes(op.op);
+  A.op = op.op; A.nplanes = workspace_planes(c, op, S, jac_mode);
   if (c.degree >= 2) p2_matrix_init(c, A, op);
   else if (A.vals.n != (size_t)A.nplanes * c.nslots) A.vals.alloc((size_t)A.nplanes * c.nslots);
   assemble_jacobian(c, op, u, A, jac_mode, eps);

@@ -180,6 +180,7 @@ SweepPrec& state(Solver& S) {
 } // namespace
 
 void ssor_setup(Ctx& c, Solver& S, const Matrix& A) {
+  PNP_REQUIRE(A.nplanes != PNP_COMPACT_PLANES, PNP_E_ARG, "SSOR sweeps 7-plane PNP matrices only");
   SweepPrec& W = state(S);
   const int F = A.nplanes == 1 ? 1 : 3;
   if (!W.plan_ssor || W.plan_ssor->F != F || W.plan_ssor->n != (long)F * c.n_own) W.plan_ssor = build_plan(c, F, false);
@@ -197,6 +198,7 @@ void ssor_apply(Ctx& c, Solver& S, const Matrix& A, const double* d, double* y) 
 }
 
 void ilu0_setup(Ctx& c, Solver& S, const Matrix& A) {
+  PNP_REQUIRE(A.nplanes != PNP_COMPACT_PLANES, PNP_E_ARG, "ILU0 factors 7-plane PNP matrices only");
   SweepPrec& W = state(S);
   const int F = A.nplanes == 1 ? 1 : 3;
   if (!W.plan_ilu || W.plan_ilu->F != F || W.plan_ilu->n != (long)F * c.n_own) W.plan_ilu = build_plan(c, F, true);

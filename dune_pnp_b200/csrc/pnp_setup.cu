@@ -474,6 +474,7 @@ void matrix_export(Ctx& c, int op_handle, const Matrix& A, double* val) {
   const Operator& op = c.oper(op_handle);
   PNP_REQUIRE(A.op == op.op, PNP_E_ARG, "matrix belongs to another operator type");
   if (c.degree >= 2) { PNP_REQUIRE(A.csr_rp, PNP_E_ARG, "matrix not assembled"); A.vals.download(val, A.csr_nnz, c.stream); return; }
+  PNP_REQUIRE(A.nplanes == op_planes(op.op), PNP_E_ARG, "matrix export reads the 7-plane PNP layout only");
   HostStar h = fetch_star(c);
   std::vector<double> v = A.vals.to_host(c.stream);
   const long ns = c.nslots;

@@ -1,6 +1,6 @@
 // pnp_spmv.cuh -- the one SpMV kernel of the library (Krylov products and every AMG level operation).
 //
-// y = A x on the star / plane layout with a fused epilogue.  HBM-bound: per launch it streams NP value planes and
+// y = A x on the star / plane layout (NP = 1, 5 or 7 value planes) with a fused epilogue.  HBM-bound: per launch it streams NP value planes and
 // the column index of every slot once ((8*NP+4)*nslots bytes), the row pointers (4*nv) and writes y (8*F*nv); x is
 // gathered (8*F*nv if every entry is fetched from DRAM once -- the locality renumbering keeps the gathers in L1/L2).
 //
@@ -33,6 +33,15 @@ constexpr int SPMV_LANES = 8;
 
 template <int NP> struct SlotData { double v[NP]; unsigned c; };
 
+// acc += B x for the 3x3 block of one slot (NP = 5 or 7 value planes, pnp_block())
+template <int NP>
+__device__ __forceinline__ void block_mac(const double* v, const double* x, double* acc) {
+  const PnpBlock B = pnp_block<NP>(v);
+  acc[0] += B.a * x[0] + B.b * x[1] + B.c * x[2];
+  acc[1] += B.d * x[0] + B.e * x[1];
+  acc[2] += B.f * x[0] + B.g * x[2];
+}
+
 template <int NP>
 __device__ __forceinline__ void load_slot(const StarOpArgs& a, int s, bool ok, SlotData<NP>& d) {
   if (ok) {
@@ -51,10 +60,8 @@ __device__ __forceinline__ void accumulate(const StarOpArgs& a, const SlotData<N
   if (NP == 1) acc[0] += d.v[0] * a.x[d.c];
   else {
     const long c = d.c;
-    const double x0 = a.x[3 * c], x1 = a.x[3 * c + 1], x2 = a.x[3 * c + 2];
-    acc[0] += d.v[0] * x0 + d.v[1 % NP] * x1 + d.v[2 % NP] * x2;
-    acc[1] += d.v[3 % NP] * x0 + d.v[4 % NP] * x1;
-    acc[2] += d.v[5 % NP] * x0 + d.v[6 % NP] * x2;
+    const double x[3] = {a.x[3 * c], a.x[3 * c + 1], a.x[3 * c + 2]};
+    block_mac<NP>(d.v, x, acc);
   }
 }
 
@@ -203,6 +210,7 @@ template <int EPI, int NDOT>
 inline int launch_star_op(Ctx& c, int nplanes, const StarOpArgs& a) {
   const int grid = star_op_grid(c, a.nv);
   if (nplanes == 1) k_star_op<1, EPI, NDOT><<<grid, SPMV_BLOCK, 0, c.stream>>>(a);
+  else if (nplanes == PNP_COMPACT_PLANES) k_star_op<PNP_COMPACT_PLANES, EPI, NDOT><<<grid, SPMV_BLOCK, 0, c.stream>>>(a);
   else k_star_op<7, EPI, NDOT><<<grid, SPMV_BLOCK, 0, c.stream>>>(a);
   PNP_CHECK_LAUNCH(); c.launches++;
   return grid;

@@ -74,10 +74,12 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned by
                ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
 
-// inverse of the diagonal block B = [a b c; d e 0; f 0 g] (planes 0..6 of the diagonal slot), row `k`; the same rule as
-// k_dinv (pnp_amg.cu): a (near-)singular block falls back to the scalar diagonal
+// inverse of the diagonal block B = [a b c; d e 0; f 0 g] (pnp_block() of the diagonal slot's NP planes), row `k`; the
+// same rule as k_dinv (pnp_amg.cu): a (near-)singular block falls back to the scalar diagonal
+template <int NP>
 __device__ __forceinline__ void block_inverse_row(const double* dv, int k, double* o) {
-  const double a = dv[0], b = dv[1], c_ = dv[2], d = dv[3], e = dv[4], f = dv[5], g = dv[6];
+  const PnpBlock B = pnp_block<NP>(dv);
+  const double a = B.a, b = B.b, c_ = B.c, d = B.d, e = B.e, f = B.f, g = B.g;
   const double det = a * e * g - b * d * g - c_ * e * f;
   const double scale = fabs(a * e * g) + fabs(b * d * g) + fabs(c_ * e * f);
   if (fabs(det) > 1e-12 * scale && scale > 0.0) {
@@ -109,12 +111,8 @@ __device__ __forceinline__ void slot_product(const StarOpArgs& a, bool ok, int s
 #pragma unroll
     for (int p = 0; p < NP; p++) dg[p] = v[p];
   }
-  if (NP == 1) acc[0] += v[0] * x[0];
-  else {
-    acc[0] += v[0] * x[0] + v[1 % NP] * x[1 % F] + v[2 % NP] * x[2 % F];
-    acc[1 % F] += v[3 % NP] * x[0] + v[4 % NP] * x[1 % F];
-    acc[2 % F] += v[5 % NP] * x[0] + v[6 % NP] * x[2 % F];
-  }
+  if constexpr (NP == 1) acc[0] += v[0] * x[0];
+  else block_mac<NP>(v, x, acc);
 }
 
 template <int NP, int EPI, int NDOT, int LPR>
@@ -273,12 +271,8 @@ __global__ void __launch_bounds__(tma_threads(NP, EPI, NDOT, LPR), 1) k_star_op_
 #pragma unroll
             for (int p = 0; p < NP; p++) dg[p] = v[p];
           }
-          if (NP == 1) acc[0] += v[0] * xj[u][0];
-          else {
-            acc[0] += v[0] * xj[u][0] + v[1 % NP] * xj[u][1 % F] + v[2 % NP] * xj[u][2 % F];
-            acc[1 % F] += v[3 % NP] * xj[u][0] + v[4 % NP] * xj[u][1 % F];
-            acc[2 % F] += v[5 % NP] * xj[u][0] + v[6 % NP] * xj[u][2 % F];
-          }
+          if constexpr (NP == 1) acc[0] += v[0] * xj[u][0];
+          else block_mac<NP>(v, xj[u], acc);
         }
         for (int j = sub + MAXS * LPR; j < maxlen; j += LPR) // rows with more slots (valence > 7)
           slot_product<NP, true>(a, j < len, b0 + j, sv, vb, sc, cbase, sx, wlo, wn, acc, nullptr);
@@ -312,12 +306,12 @@ __global__ void __launch_bounds__(tma_threads(NP, EPI, NDOT, LPR), 1) k_star_op_
           double r[F], z[F];
 #pragma unroll
           for (int k = 0; k < F; k++) r[k] = sb[F * rl + k] - acc[k];
-          if (F == 3) {
+          if constexpr (F == 3) {
 #pragma unroll
             for (int k = 0; k < F; k++) {
               double o[3];
-              block_inverse_row(dg, k, o);
-              z[k] = o[0] * r[0] + o[1] * r[1 % F] + o[2] * r[2 % F];
+              block_inverse_row<NP>(dg, k, o);
+              z[k] = o[0] * r[0] + o[1] * r[1] + o[2] * r[2];
             }
           } else z[0] = (dg[0] != 0.0 ? 1.0 / dg[0] : 0.0) * r[0];
 #pragma unroll
@@ -416,7 +410,9 @@ inline int launch_star_op_auto(Ctx& c, int nplanes, const StarOpArgs& a, bool fi
   c.acct(fine ? Ctx::ACC_SPMV_FINE : Ctx::ACC_SPMV_COARSE, star_op_bytes<EPI, NDOT>(nplanes, a));
   if (EPI != EPI_CHEBYSHEV && star_op_tma_ok(c, a, EPI)) {
     constexpr int E = EPI == EPI_CHEBYSHEV ? EPI_PLAIN : EPI; // (never instantiated for Chebyshev)
-    return nplanes == 1 ? launch_star_op_tma_inst<1, E, NDOT>(c, a) : launch_star_op_tma_inst<7, E, NDOT>(c, a);
+    return nplanes == 1 ? launch_star_op_tma_inst<1, E, NDOT>(c, a)
+         : nplanes == PNP_COMPACT_PLANES ? launch_star_op_tma_inst<PNP_COMPACT_PLANES, E, NDOT>(c, a)
+                                         : launch_star_op_tma_inst<7, E, NDOT>(c, a);
   }
   return launch_star_op<EPI, NDOT>(c, nplanes, a);
 }

@@ -11,7 +11,7 @@
 //                  and with it the reference's quadrature/summation order, can be reconstructed)
 //   STAR_CW      : the element is stored clockwise (then next-in-ring is its cyclic successor)
 // Vectors are vertex-blocked: dof (v, field k) lives at F*v + k.  Matrix values are stored as
-// NPLANES planes of nslots doubles (PNP: 7 planes, see pnp_plane()).
+// NPLANES planes of nslots doubles (PNP: 7 planes, see pnp_plane(), or the compact 5, see pnp_block()).
 //
 // This replaces PDELab's element loop + scatter (GridOperator::residual/jacobian, SURVEY App. A.2;
 // call sites /root/reference/src/stationary_pnp.hh:240-246): every residual entry / matrix slot is
@@ -122,21 +122,31 @@ PNP_HD void residual_row(const StarView& M, const PhysParams& P, const double* u
 // ---- Jacobian ------------------------------------------------------------------------------
 enum : int { JAC_FD_FAITHFUL = 0, JAC_ANALYTIC = 1 };
 
-template <int OP, int I, int MODE>
+template <int OP, int I, int MODE, int NP>
 PNP_HD void tri_jac(const VData<OP>& A0, const VData<OP>& A1, const VData<OP>& A2, const PhysParams& P, double eps,
-                    double (*blk)[OpTraits<OP>::NPLANES]) {
+                    double (*blk)[NP]) {
   double xl[VData<OP>::F][3], aux[VData<OP>::NA][3];
   const Geo G = gather_local<OP>(A0, A1, A2, xl, aux);
-  if (MODE == JAC_FD_FAITHFUL) jac_rows_fd<OP, I>(G, P, xl, aux, eps, blk);
+  if constexpr (NP != OpTraits<OP>::NPLANES) {
+    static_assert(OP == OP_PNP && NP == PNP_COMPACT_PLANES && MODE == JAC_ANALYTIC, "compact layout: exact PNP Jacobian only");
+    jac_rows_exact_compact<I>(G, P, xl, blk);
+  } else if (MODE == JAC_FD_FAITHFUL) jac_rows_fd<OP, I>(G, P, xl, aux, eps, blk);
   else jac_rows_exact<OP, I>(G, P, xl, aux, blk);
 }
 
 // Dirichlet treatment of one block (SURVEY App. A.2): entries whose row or column dof is
 // constrained are dropped; a constrained row keeps a unit diagonal.  rb/cb = Dirichlet bits of the
-// row/column vertex restricted to this operator's fields.
-template <int OP>
+// row/column vertex restricted to this operator's fields.  The compact layout's vertices are constrained in all three
+// fields or in none (pnp_jacobian_planes): the block goes as a whole, a constrained row keeps L = 1, D = 0.
+template <int OP, int NP = OpTraits<OP>::NPLANES>
 PNP_HD void mask_block(double* b, unsigned rb, unsigned cb, bool diagonal) {
-  if (OP == OP_PNP) {
+  if (NP == PNP_COMPACT_PLANES) {
+    if ((rb | cb) & 7u) {
+#pragma unroll
+      for (int p = 0; p < NP; p++) b[p] = 0.0;
+      if (diagonal && (rb & 1u)) b[0] = 1.0;
+    }
+  } else if (OP == OP_PNP) {
 #pragma unroll
     for (int ki = 0; ki < 3; ki++)
 #pragma unroll
@@ -158,11 +168,10 @@ template <int OP> PNP_HD unsigned dir_bits(const StarView& M, int w, int comp0) 
 }
 
 // Assembles the block row of vertex v into vals[plane*stride + slot - sbase] (sbase != 0: `vals` is a staging tile
-// that starts at global slot sbase).
-template <int OP, int MODE>
+// that starts at global slot sbase), in the operator's NPLANES planes or, NP = PNP_COMPACT_PLANES, the compact layout.
+template <int OP, int MODE, int NP = OpTraits<OP>::NPLANES>
 PNP_HD void jacobian_row(const StarView& M, const PhysParams& P, const double* u, const double* aux0,
                          const double* aux1, double eps, int comp0, int v, double* vals, long stride, int sbase = 0) {
-  constexpr int NP = OpTraits<OP>::NPLANES;
   vals -= sbase; // only entries [sbase, ...) of a plane are touched
   const int sd = M.rp[v], s0 = sd + 1, s1 = M.rp[v + 1];
   const unsigned rb = dir_bits<OP>(M, v, comp0);
@@ -196,7 +205,7 @@ PNP_HD void jacobian_row(const StarView& M, const PhysParams& P, const double* u
           for (int p = 0; p < NP; p++) blk[j][p] = 0.0;
         const double *bv, *bcur, *bnxt;
         if (MODE == JAC_ANALYTIC) { // vertex-centric order (v, this neighbour, next neighbour): no branch on li
-          tri_jac<OP, 0, MODE>(V, cur, nxt, P, eps, blk);
+          tri_jac<OP, 0, MODE, NP>(V, cur, nxt, P, eps, blk);
           bv = blk[0]; bcur = blk[1]; bnxt = blk[2];
         } else {
           const int li = (a_cur >> STAR_LI_SHIFT) & 3;
@@ -205,9 +214,9 @@ PNP_HD void jacobian_row(const StarView& M, const PhysParams& P, const double* u
           const VData<OP>& Pp = cw ? cur : nxt;
           // local column index of: v -> li, n -> (li+1)%3, p -> (li+2)%3
           const double *bn, *bp;
-          if (li == 0) { tri_jac<OP, 0, MODE>(V, N, Pp, P, eps, blk); bv = blk[0]; bn = blk[1]; bp = blk[2]; }
-          else if (li == 1) { tri_jac<OP, 1, MODE>(Pp, V, N, P, eps, blk); bv = blk[1]; bn = blk[2]; bp = blk[0]; }
-          else { tri_jac<OP, 2, MODE>(N, Pp, V, P, eps, blk); bv = blk[2]; bn = blk[0]; bp = blk[1]; }
+          if (li == 0) { tri_jac<OP, 0, MODE, NP>(V, N, Pp, P, eps, blk); bv = blk[0]; bn = blk[1]; bp = blk[2]; }
+          else if (li == 1) { tri_jac<OP, 1, MODE, NP>(Pp, V, N, P, eps, blk); bv = blk[1]; bn = blk[2]; bp = blk[0]; }
+          else { tri_jac<OP, 2, MODE, NP>(N, Pp, V, P, eps, blk); bv = blk[2]; bn = blk[0]; bp = blk[1]; }
           bcur = cw ? bp : bn;
           bnxt = cw ? bn : bp;
         }
@@ -219,7 +228,7 @@ PNP_HD void jacobian_row(const StarView& M, const PhysParams& P, const double* u
         for (int p = 0; p < NP; p++) carry[p] = 0.0;
       }
       if (!(last && closed && s == s0)) { // (a one-slot closed ring cannot exist)
-        mask_block<OP>(val, rb, cb_cur, false);
+        mask_block<OP, NP>(val, rb, cb_cur, false);
 #pragma unroll
         for (int p = 0; p < NP; p++) vals[p * stride + s] = val[p];
       }
@@ -227,14 +236,27 @@ PNP_HD void jacobian_row(const StarView& M, const PhysParams& P, const double* u
       cb_cur = last ? cb_first : dir_bits<OP>(M, (int)(a_nxt & STAR_VMASK), comp0);
     }
     if (closed) { // the wrap-around triangle's contribution to the first ring slot
-      mask_block<OP>(carry, rb, cb_first, false);
+      mask_block<OP, NP>(carry, rb, cb_first, false);
 #pragma unroll
       for (int p = 0; p < NP; p++) vals[p * stride + s0] += carry[p];
     }
   }
-  mask_block<OP>(diag, rb, rb, true);
+  mask_block<OP, NP>(diag, rb, rb, true);
 #pragma unroll
   for (int p = 0; p < NP; p++) vals[p * stride + sd] = diag[p];
+}
+
+// Value planes of a PNP Jacobian that only the star SpMV and diagonal-block consumers read (solver_ok: no SSOR / ILU0 /
+// Gauss-Seidel sweeps): the compact layout for the exact derivative on linear elements when every surface of the
+// parameter set has its three components all Dirichlet or all not (btype: 3 per surface, 0 = Dirichlet); else 7.
+// Decided from the parameters alone, so every rank of a partitioned mesh takes the same layout.
+inline int pnp_jacobian_planes(int mode, int degree, bool solver_ok, const int* btype, int n_surfaces) {
+  if (mode != JAC_ANALYTIC || degree != 1 || !solver_ok) return OpTraits<OP_PNP>::NPLANES;
+  for (int s = 0; s < n_surfaces; s++) {
+    const bool d0 = btype[3 * s] == 0;
+    if ((btype[3 * s + 1] == 0) != d0 || (btype[3 * s + 2] == 0) != d0) return OpTraits<OP_PNP>::NPLANES;
+  }
+  return PNP_COMPACT_PLANES;
 }
 
 // ---- boundary term (alpha_boundary) -------------------------------------------------------------

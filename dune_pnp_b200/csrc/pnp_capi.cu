@@ -10,6 +10,7 @@ int newton_apply(Ctx&, const Operator&, Vec&, Solver&, const pnp_newton_opts&, p
 int amg_graph_state(const Solver&); // pnp_amg.cu
 LinResult slp_apply(Ctx&, const Operator&, Vec&, Solver&, double, int, double);
 int onestep_apply(Ctx&, int, const Operator&, const Operator&, Solver&, double, Vec&, Vec&, Vec&, double, int, double, LinResult*);
+int pnp_context_planes(const Ctx&, int jac_mode, bool solver_ok); // pnp_newton.cu
 namespace {
 __global__ void k_fill(double* x, long n, double v) {
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) x[i] = v;
@@ -232,6 +233,7 @@ pnp_status pnp_tune(const char* name, double value) {
   else if (n == "graph") t.graph = value != 0;
   else if (n == "fd_warp") t.fd_warp = value != 0;
   else if (n == "jac_compact") t.jac_compact = value != 0;
+  else if (n == "matrix_compact") t.matrix_compact = value != 0;
   else if (n == "p2_chunk") t.p2_chunk = (long)value;
   else if (n == "tma_min_rows") t.tma_min_rows = (long)value;
   else return PNP_E_ARG;
@@ -490,6 +492,7 @@ pnp_status pnp_matrix_create(pnp_ctx* ctx, int op_handle, int* handle) {
   PNP_REQUIRE(c.finalized && handle, PNP_E_ARG, "mesh not finalized");
   auto m = std::make_unique<Matrix>();
   m->op = c.oper(op_handle).op; m->nplanes = op_planes(m->op);
+  if (m->op == OP_PNP && tune().matrix_compact) m->nplanes = pnp_context_planes(c, JAC_ANALYTIC, true);
   if (c.degree >= 2) { PNP_REQUIRE(c.constraints_built, PNP_E_ARG, "constraints not built"); p2_matrix_init(c, *m, c.oper(op_handle)); }
   else { m->vals.alloc((size_t)m->nplanes * c.nslots); m->vals.zero(c.stream); }
   c.mats.push_back(std::move(m));

@@ -71,6 +71,7 @@ struct Tune {
   int graph = 1;          // the multigrid's coarse correction is replayed from a CUDA graph
   int fd_warp = 1;        // FD-faithful Jacobian: warp-cooperative kernel (0: one thread per vertex)
   int jac_compact = 1;    // Newton / linear-problem Jacobian in the compact 5-plane PNP layout where it applies (0: always 7)
+  int matrix_compact = 0; // pnp_matrix_create: PNP matrices in the compact layout where the exact Jacobian has it (0: always 7)
   long p2_chunk = 0;      // quadratic / cubic elements: elements per scratch block of the Jacobian assembly (0: 2 GB worth)
 };
 inline Tune& tune() { static Tune t; return t; }

@@ -12,6 +12,15 @@
 
 namespace pnp {
 
+// Value planes of a PNP Jacobian of this context (pnp_jacobian_planes of its parameter set): the compact layout needs one
+// unpartitioned GPU mesh.
+int pnp_context_planes(const Ctx& c, int jac_mode, bool solver_ok) {
+  if (c.n_own != c.nv || !c.mg.empty()) return op_planes(OP_PNP);
+  std::vector<int> btype;
+  for (const HostSurface& s : c.params.surfaces) btype.insert(btype.end(), s.btype, s.btype + 3);
+  return pnp_jacobian_planes(jac_mode, c.degree, solver_ok, btype.data(), (int)c.params.surfaces.size());
+}
+
 namespace {
 double now() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
@@ -19,12 +28,10 @@ double now() { return std::chrono::duration<double>(std::chrono::steady_clock::n
 // through star SpMVs and diagonal blocks only -- no preconditioner, Jacobi, or the multigrid with the Jacobi or Chebyshev
 // smoother -- on one GPU.  Everything else keeps the operator's planes.
 int workspace_planes(const Ctx& c, const Operator& op, const Solver& S, int jac_mode) {
-  if (op.op != OP_PNP || !tune().jac_compact || c.n_own != c.nv || !c.mg.empty()) return op_planes(op.op);
+  if (op.op != OP_PNP || !tune().jac_compact) return op_planes(op.op);
   const double sm = S.opt("amg_smoother", 0);
   const bool solver_ok = S.prec == PNP_PREC_NONE || S.prec == PNP_PREC_JACOBI || (S.prec == PNP_PREC_AMG && (sm == 0 || sm == 1));
-  std::vector<int> btype;
-  for (const HostSurface& s : c.params.surfaces) btype.insert(btype.end(), s.btype, s.btype + 3);
-  return pnp_jacobian_planes(jac_mode, c.degree, solver_ok, btype.data(), (int)c.params.surfaces.size());
+  return pnp_context_planes(c, jac_mode, solver_ok);
 }
 } // namespace
 

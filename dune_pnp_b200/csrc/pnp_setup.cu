@@ -474,10 +474,15 @@ void matrix_export(Ctx& c, int op_handle, const Matrix& A, double* val) {
   const Operator& op = c.oper(op_handle);
   PNP_REQUIRE(A.op == op.op, PNP_E_ARG, "matrix belongs to another operator type");
   if (c.degree >= 2) { PNP_REQUIRE(A.csr_rp, PNP_E_ARG, "matrix not assembled"); A.vals.download(val, A.csr_nnz, c.stream); return; }
-  PNP_REQUIRE(A.nplanes == op_planes(op.op), PNP_E_ARG, "matrix export reads the 7-plane PNP layout only");
   HostStar h = fetch_star(c);
   std::vector<double> v = A.vals.to_host(c.stream);
   const long ns = c.nslots;
+  if (A.nplanes == PNP_COMPACT_PLANES) { // expanded as the solver kernels read it: (c+,c+) = L - D, (c-,c-) = L + D, ...
+    walk_pattern(c, op, h, nullptr, [&](long k, int ki, int kj, int slot, bool) {
+      val[k] = pnp_block_at<PNP_COMPACT_PLANES>(v.data(), ns, slot).at(ki, kj);
+    });
+    return;
+  }
   walk_pattern(c, op, h, nullptr, [&](long k, int ki, int kj, int slot, bool) {
     int pl = op.op == OP_PNP ? pnp_plane(ki, kj) : 0;
     val[k] = pl < 0 ? 0.0 : v[(size_t)pl * ns + slot];
@@ -495,6 +500,8 @@ void matrix_import(Ctx& c, int op_handle, Matrix& A, const int* rowptr, const in
   const Operator& op = c.oper(op_handle);
   PNP_REQUIRE(A.op == op.op, PNP_E_ARG, "matrix belongs to another operator type");
   if (c.degree >= 2) { p2_matrix_import(c, op, A, rowptr, col, val); return; }
+  // an arbitrary CSR matrix has no compact form (its diagonal blocks need not share one Laplacian)
+  PNP_REQUIRE(A.nplanes == op_planes(op.op), PNP_E_ARG, "matrix import writes the 7-plane PNP layout only");
   HostStar h = fetch_star(c);
   const long ns = c.nslots, nv = c.nv;
   std::vector<double> v((size_t)A.nplanes * ns, 0.0);

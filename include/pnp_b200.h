@@ -54,7 +54,9 @@ const char* pnp_last_error(pnp_ctx* ctx);
 /* process-wide kernel tuning knobs (experiments, tests): "tma" (1: large levels run the bulk-copy streaming SpMV, 0: the
  * plain-load kernel everywhere), "tma_stages" (2..3), "tma_min_rows" (smallest level served by the streaming kernel, -1:
  * two tiles per SM), "tma_lpr" (lanes per row, 1 or 2), "graph" (1: the multigrid's coarse correction is replayed from a
- * CUDA graph) */
+ * CUDA graph), "matrix_compact" (1: pnp_matrix_create gives PNP matrices the compact 5-plane layout where the exact
+ * Jacobian has it -- linear elements, every surface constraining all three fields or none, one unpartitioned mesh;
+ * pnp_matrix_set_csr, FD assembly, SSOR, ILU0 and the Gauss-Seidel smoother refuse such a matrix) */
 pnp_status pnp_tune(const char* name, double value);
 /* number of CUDA kernels this context has launched so far */
 long pnp_launch_count(pnp_ctx* ctx);

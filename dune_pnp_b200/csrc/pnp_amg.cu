@@ -42,6 +42,13 @@ struct Level {
   const int* rp = nullptr; const unsigned* col = nullptr; const double* vals = nullptr;
   DBuf<int> rp_own; DBuf<unsigned> col_own; DBuf<double> vals_own;
   DBuf<double> dinv, x, x2, b, r;
+  // single-precision companion of `vals` (empty: none, mg_f32_rule()): the same planes rounded to nearest, stride32 (a
+  // multiple of 4) floats apart so that every plane starts on a 16-byte boundary.  Where it exists, every operation of
+  // the smoothing cycle on this level -- the first Jacobi sweep's stored block inverses, the smoother steps and the
+  // residual -- applies the rounded matrix (widened to double); the Krylov operator, the Galerkin products, the dense
+  // coarsest level and the exports keep reading `vals`.  Rebuilt from `vals` by every numeric set-up, never written
+  // anywhere else, so it cannot go stale when the caller's planes change.
+  DBuf<float> vals32; long stride32 = 0;
   double lmax = 2.0;      // Gershgorin bound of the spectrum of D^-1 A
   // transfer to the next coarser level
   // Prolongation row of fine vertex i: one parent (weight 1: aggregate / coinciding coarse vertex) or two parents
@@ -87,6 +94,7 @@ struct Amg {
   DBuf<double> dense, dense_work;
   DBuf<int> dense_piv, dense_info;
   bool distributed = false; // levels are parts of a mesh hierarchy spread over the ranks (halo exchange per level)
+  bool replica = false;     // the single-GPU hierarchy below a distributed one's replicated coarsest level (rep_solver)
   bool redisc = false;      // one GPU: the geometric levels are re-discretised (as the distributed levels are), not Galerkin products
   DBuf<double> grhs;        // replicated coarsest level: global right-hand side / solution
   // replica variant (Ctx::mg_replica): the coarsest distributed level is gathered to a context that holds the whole
@@ -263,15 +271,18 @@ __global__ void k_galerkin(const int* __restrict__ seg_ptr, const int* __restric
 // smoother matrix M^-1: scalar operators 1/a_ii; PNP: inverse of every vertex's 3x3 diagonal block (point-block Jacobi --
 // the phi/c couplings inside a vertex grow like h^2 relative to the stiffness terms, so on coarse levels a scalar
 // diagonal no longer dominates them)
-template <int NP>
-__global__ void k_dinv(const int* __restrict__ rp, const double* __restrict__ vals, long stride, int nv,
+template <int NP, class T>
+__global__ void k_dinv(const int* __restrict__ rp, const T* __restrict__ vals, long stride, int nv,
                        double* __restrict__ dinv) {
   for (int v = blockIdx.x * blockDim.x + threadIdx.x; v < nv; v += gridDim.x * blockDim.x) {
     const int s = rp[v];
     if (NP == 1) { const double d = vals[s]; dinv[v] = d != 0.0 ? 1.0 / d : 0.0; }
     else {
-      // B = [a b c; d e 0; f 0 g]
-      const PnpBlock B = pnp_block_at<NP>(vals, stride, s);
+      // B = [a b c; d e 0; f 0 g] (float planes widened first: the block of the rounded matrix, inverted in double)
+      double pv[NP];
+#pragma unroll
+      for (int p = 0; p < NP; p++) pv[p] = vals[p * stride + s];
+      const PnpBlock B = pnp_block<NP>(pv);
       const double a = B.a, b = B.b, c_ = B.c, d = B.d, e = B.e, f = B.f, g = B.g;
       const double det = a * e * g - b * d * g - c_ * e * f;
       double* o = dinv + 9l * v;
@@ -287,6 +298,13 @@ __global__ void k_dinv(const int* __restrict__ rp, const double* __restrict__ va
       }
     }
   }
+}
+// single-precision companion of a level's planes: o[p * stride32 + s] = fl32(v[p * stride + s]), zero in the padding
+__global__ void k_round_planes(const double* __restrict__ v, long stride, long ns, float* __restrict__ o, long stride32) {
+  const double* vp = v + blockIdx.y * stride;
+  float* op = o + blockIdx.y * stride32;
+  for (long s = blockIdx.x * (long)blockDim.x + threadIdx.x; s < stride32; s += (long)gridDim.x * blockDim.x)
+    op[s] = s < ns ? __double2float_rn(vp[s]) : 0.0f;
 }
 // first sweep from a zero initial guess: x = omega * M^-1 b  (also the first Chebyshev direction d)
 template <int F>
@@ -505,6 +523,7 @@ void level_op(Ctx& c, const Amg& A, const Level& l, const double* x, const doubl
               double c1 = 0.0, double* dvec = nullptr) {
   StarOpArgs a{l.rp, l.col, l.vals, l.nslots, l.nv, x, y};
   a.b = b; a.dinv = l.dinv.p; a.block = A.F == 3; a.omega = omega_or_c2 < 0 ? A.omega : omega_or_c2; a.c1 = c1; a.dvec = dvec;
+  a.vals32 = l.vals32.p; a.stride32 = l.stride32; // (the one place that picks the planes a cycle operation reads)
   const bool fine = &l == A.L[0].get();
   if (A.distributed) halo_exchange(*l.lc, const_cast<double*>(x), A.F); // ghost columns of the iterate
   if (fine) c.prof_mark(EPI == EPI_RESIDUAL ? 1 : 2);
@@ -720,11 +739,46 @@ const double* level_values(Ctx& c, Amg& A, int li, const double* uf, int comp0) 
   return nullptr;
 }
 
-// smoother matrix of level l (k_dinv)
+// smoother matrix of level l (k_dinv): from the planes the level's cycle operations read
+template <class T>
+void level_dinv_t(Ctx& c, Amg& A, Level& l, const T* vals, long stride) {
+  if (A.NP == 1) KL(c, (k_dinv<1, T>), l.nv, l.rp, vals, stride, l.nv, l.dinv.p);
+  else if (A.NP == PNP_COMPACT_PLANES) KL(c, (k_dinv<PNP_COMPACT_PLANES, T>), l.nv, l.rp, vals, stride, l.nv, l.dinv.p);
+  else KL(c, (k_dinv<7, T>), l.nv, l.rp, vals, stride, l.nv, l.dinv.p);
+  c.acct(Ctx::ACC_ASSEMBLY, (4.0 + sizeof(T) * A.NP + (A.F == 3 ? 72.0 : 8.0)) * l.nv);
+}
 void level_dinv(Ctx& c, Amg& A, Level& l) {
-  if (A.NP == 1) KL(c, k_dinv<1>, l.nv, l.rp, l.vals, l.nslots, l.nv, l.dinv.p);
-  else if (A.NP == PNP_COMPACT_PLANES) KL(c, k_dinv<PNP_COMPACT_PLANES>, l.nv, l.rp, l.vals, l.nslots, l.nv, l.dinv.p);
-  else KL(c, k_dinv<7>, l.nv, l.rp, l.vals, l.nslots, l.nv, l.dinv.p);
+  if (l.vals32.p) level_dinv_t<float>(c, A, l, l.vals32.p, l.stride32);
+  else level_dinv_t<double>(c, A, l, l.vals, l.nslots);
+}
+
+// Which levels smooth against a single-precision companion of their matrix: one GPU (no partitioned or replicated
+// hierarchy), damped Jacobi, a level the streaming SpMV serves, and at least mg_f32_min_rows rows (pnp_tune; -1: 2^22).
+// The smoother and the residual of such a level read 4 bytes less per plane and slot (0.64x the bytes of a
+// compact-layout pass); the multigrid is only a preconditioner, and the Krylov method keeps applying the fp64 matrix,
+// so the accuracy a solve can reach is unchanged.  The default puts levels 7 and 6 of the pore mesh (47.1 M and 11.8 M
+// vertices) on the float side; level 5 (2.9 M) and below, ~1 % of the step's bytes, stay in double, so that the
+// cycle's corrections of the 5- and 7-plane layouts agree to rounding at those sizes.
+bool mg_f32_rule(Ctx& c, const Amg& A, Level& l) {
+  if (A.distributed || A.replica || A.smoother != 0) return false;
+  const long t = tune().mg_f32_min_rows;
+  if ((long)l.nv < (t >= 0 ? t : (1l << 22))) return false;
+  StarOpArgs a{l.rp, l.col, l.vals, l.nslots, l.nv, l.x.p, l.x2.p};
+  a.b = l.r.p;
+  return star_op_tma_ok(c, a, EPI_JACOBI);
+}
+// (re)builds or drops level l's companion; true if the planes its cycle reads changed place
+bool level_f32(Ctx& c, Amg& A, Level& l) {
+  float* before = l.vals32.p;
+  if (!mg_f32_rule(c, A, l)) { l.vals32.release(); l.stride32 = 0; return before != nullptr; }
+  l.stride32 = (l.nslots + 3) & ~3l;
+  const size_t n = (size_t)A.NP * l.stride32;
+  if (l.vals32.n != n) l.vals32.alloc(n);
+  const dim3 grid((unsigned)grid_for(l.stride32, BLK, 148 * 8), (unsigned)A.NP);
+  k_round_planes<<<grid, BLK, 0, c.stream>>>(l.vals, l.nslots, l.nslots, l.vals32.p, l.stride32);
+  PNP_CHECK_LAUNCH(); c.launches++;
+  c.acct(Ctx::ACC_ASSEMBLY, (8.0 * l.nslots + 4.0 * l.stride32) * A.NP);
+  return before != l.vals32.p;
 }
 
 // Gershgorin bounds of D^-1 A on every level (Chebyshev smoother); distributed: the maximum over the ranks
@@ -765,22 +819,20 @@ void numeric(Ctx& c, Amg& A, int comp0) {
       c.absorb(*n.lc);
       uf = n.u.d.p;
     }
-    for (size_t li = 0; li < A.L.size(); li++) {
-      Level& l = *A.L[li];
-      level_dinv(c, A, l);
-      c.acct(Ctx::ACC_ASSEMBLY, (4.0 + 8.0 * A.NP + (A.F == 3 ? 72.0 : 8.0)) * l.nv);
-    }
+    for (size_t li = 0; li < A.L.size(); li++) level_dinv(c, A, *A.L[li]);
     if (c.mg_replica) replica_setup(c, A); else dense_factor_global(c, A);
     if (A.smoother == 1) gershgorin_bounds(c, A);
     return;
   }
   const double* uf = c.last_u;
+  bool moved = false;
   for (size_t li = 0; li < A.L.size(); li++) {
     Level& l = *A.L[li];
     if (li + 1 < A.L.size()) uf = level_values(c, A, (int)li, uf, comp0);
+    moved |= level_f32(c, A, l) && li > 0; // (level l's fp64 values are final here)
     level_dinv(c, A, l);
-    c.acct(Ctx::ACC_ASSEMBLY, (4.0 + 8.0 * A.NP + (A.F == 3 ? 72.0 : 8.0)) * l.nv);
   }
+  if (moved) A.cg_reset(); // the captured coarse correction names the planes its launches read
   A.dense_n = 0;
   if ((long)A.F * A.L.back()->nv <= A.dense_max) dense_factor(c, A); // (a one-level hierarchy is a direct solve)
   if (A.smoother == 1) gershgorin_bounds(c, A);
@@ -921,7 +973,10 @@ void replica_setup(Ctx& c, Amg& A) {
   if (A.rep_A.vals.n != (size_t)A.NP * rc.nslots) A.rep_A.vals.alloc((size_t)A.NP * rc.nslots);
   rc.launches = 0;
   assemble_jacobian(rc, op, A.rep_u, A.rep_A, c.last_mode, c.last_eps);
-  if (!A.rep_solver) { A.rep_solver = std::make_unique<Solver>(); A.rep_solver->prec = PNP_PREC_AMG; }
+  if (!A.rep_solver) {
+    A.rep_solver = std::make_unique<Solver>(); A.rep_solver->prec = PNP_PREC_AMG;
+    A.rep_solver->amg = std::make_shared<Amg>(); A.rep_solver->amg->replica = true;
+  }
   auto& ro = A.rep_solver->opts;
   ro["amg_geometric"] = 1; /* refinement levels the replica made itself, if any */ ro["amg_omega"] = A.omega; ro["amg_alpha"] = A.alpha; ro["amg_gamma"] = A.gamma;
   ro["amg_dense_max"] = A.dense_max; ro["amg_coarse_sweeps"] = A.coarse_sweeps; ro["amg_smoother"] = A.smoother;

@@ -236,6 +236,7 @@ pnp_status pnp_tune(const char* name, double value) {
   else if (n == "matrix_compact") t.matrix_compact = value != 0;
   else if (n == "p2_chunk") t.p2_chunk = (long)value;
   else if (n == "tma_min_rows") t.tma_min_rows = (long)value;
+  else if (n == "mg_f32_min_rows") t.mg_f32_min_rows = value > 9e18 ? (long)9e18 : (long)value;
   else return PNP_E_ARG;
   return PNP_OK;
 }

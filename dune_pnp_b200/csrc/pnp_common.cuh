@@ -68,6 +68,7 @@ struct Tune {
   int tma_stages = 2;     // ring depth of the streaming SpMV (2..3); two stages leave more of the SM's memory to L1
   int tma_lpr = 2;        // lanes per row in the streaming SpMV (1 or 2): 2 -> eight consumer warps per SM
   long tma_min_rows = -1; // smallest level the streaming SpMV serves (-1: two tiles per SM)
+  long mg_f32_min_rows = -1; // smallest multigrid level smoothed against a single-precision copy of its matrix (-1: 2^22)
   int graph = 1;          // the multigrid's coarse correction is replayed from a CUDA graph
   int fd_warp = 1;        // FD-faithful Jacobian: warp-cooperative kernel (0: one thread per vertex)
   int jac_compact = 1;    // Newton / linear-problem Jacobian in the compact 5-plane PNP layout where it applies (0: always 7)

@@ -26,6 +26,9 @@ struct StarOpArgs {
   double* dvec = nullptr;         // Chebyshev direction (in/out)
   const double* w1 = nullptr;     // NDOT >= 1: partial sums of y.w1 ; NDOT == 2: also y.y
   double* partial = nullptr;
+  // the same matrix in single precision, NP planes stride32 (a multiple of 4) floats apart: when set, the streaming
+  // kernel's residual / smoother step reads these planes instead of `vals` (pnp_spmv_tma.cuh)
+  const float* vals32 = nullptr; long stride32 = 0;
 };
 
 constexpr int SPMV_BLOCK = 256;

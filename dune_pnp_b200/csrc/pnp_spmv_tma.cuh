@@ -19,6 +19,10 @@
 //
 // The damped point-block Jacobi epilogue inverts every vertex's 3x3 diagonal block from the diagonal slot that is in
 // shared memory anyway, instead of reading a stored inverse (72 B/vertex, 12 % of the smoother's traffic).
+//
+// T is the type of the stored value planes: double (StarOpArgs::vals), or float (StarOpArgs::vals32, the multigrid's
+// single-precision copy of a large level's matrix, pnp_amg.cu) for the residual and smoother epilogues.  A float value
+// is widened to double as it leaves shared memory: products, sums, the block inverse and the epilogue stay fp64.
 #pragma once
 #include "pnp_spmv.cuh"
 
@@ -29,14 +33,28 @@ constexpr int tma_nw(int lpr) { return TMA_TR * lpr / 32; } // consumer warps fo
 // producer warps: one per copy stream of a tile -- NP value planes, column indices, row pointers, x window, and the
 // right-hand side / dot operand where the epilogue reads one
 constexpr int tma_producers(int np, int epi, int ndot) { return np + 3 + ((epi != EPI_PLAIN || ndot >= 1) ? 1 : 0); }
-constexpr int tma_threads(int np, int epi, int ndot, int lpr) { return (tma_nw(lpr) + tma_producers(np, epi, ndot)) * 32; }
+// Consumer groups: with float planes a tile's bytes arrive in 0.64x the time, and one group of consumer warps -- which
+// finishes a tile, including the round trip of its out-of-window x gathers, before it starts the next -- paced the
+// kernel at 0.57 of the copy bandwidth (3.30 ms against 3.57 ms in double, k = 7, B200).  Two groups take alternate
+// tiles, so one group's gathers are in flight while the other computes.  With two groups the row pointers and the
+// right-hand side (two small copies) share a producer warp: 24 warps of the 5-plane kernel leave 80 registers a
+// thread, 25 would leave 72 and spill.  (With one lane per row two groups leave too few registers: one group.)
+template <class T> constexpr int tma_groups(int lpr) { return sizeof(T) == 4 && lpr == 2 ? 2 : 1; }
+constexpr bool tma_shared_rp_b(int np, int epi, int ndot, int groups) { return groups > 1 && tma_producers(np, epi, ndot) == np + 4; }
+constexpr int tma_threads(int np, int epi, int ndot, int lpr, int groups = 1) {
+  return (groups * tma_nw(lpr) + tma_producers(np, epi, ndot) - (tma_shared_rp_b(np, epi, ndot, groups) ? 1 : 0)) * 32;
+}
 constexpr int TMA_CAP = 960;                     // staged slots per tile and plane
-constexpr int TMA_MAX_STAGES = 3;
+constexpr int TMA_MAX_STAGES = 3;                // ring depth of the double-plane kernel (tune().tma_stages)
+constexpr int TMA_F32_STAGES = 4;                // ... of the float-plane kernel: two per consumer group
 constexpr int TMA_W = 128;                       // rows of x staged on either side of the tile (the gather window)
 
-template <int NP> struct TmaLayout {
+template <int NP, class T = double> struct TmaLayout {
   static constexpr int F = NP == 1 ? 1 : 3;
-  static constexpr int PLANE = (TMA_CAP + 2) * 8;                    // bytes of one value plane of a stage
+  // bytes of one value plane of a stage: CAP slots plus the rounding of the source down to 16 bytes (1 double: the
+  // plane-parity offset; 3 floats: float planes start on 16-byte boundaries, StarOpArgs::stride32)
+  static constexpr int PLANE = sizeof(T) == 8 ? (TMA_CAP + 2) * 8 : (TMA_CAP + 4) * 4;
+  static constexpr int PSLOTS = PLANE / (int)sizeof(T);
   static constexpr int COLS = NP * PLANE;                            // (CAP + 4) column indices
   static constexpr int RP = COLS + (TMA_CAP + 4) * 4;                // (TR + 4) row pointers
   static constexpr int B = RP + (TMA_TR + 4) * 4;                    // F*TR (+2) doubles: right-hand side / dot operand
@@ -45,8 +63,9 @@ template <int NP> struct TmaLayout {
   // from it as well
   static constexpr int XW = B + (F * TMA_TR + 2) * 8;
   static constexpr int STAGE = XW + (F * (TMA_TR + 2 * TMA_W) + 2) * 8;
-  static constexpr int YBUF = TMA_TR * F * 8;                        // output staging, per consumer warp a slice
-  static constexpr int HEAD = 128;                                   // mbarriers
+  static constexpr int YBUF = 2 * TMA_TR * F * 8;                    // output staging, per consumer warp a slice (2 groups)
+  static constexpr int HEAD = 128;                                   // mbarriers (full and empty, up to 8 stages)
+  static constexpr int MAX_STAGES = sizeof(T) == 8 ? TMA_MAX_STAGES : TMA_F32_STAGES;
   static_assert(PLANE % 16 == 0 && COLS % 16 == 0 && RP % 16 == 0 && B % 16 == 0 && XW % 16 == 0 && STAGE % 16 == 0, "bulk copy alignment");
   static constexpr int smem_bytes(int stages) { return HEAD + stages * STAGE + YBUF; }
 };
@@ -94,10 +113,16 @@ __device__ __forceinline__ void block_inverse_row(const double* dv, int k, doubl
   }
 }
 
+// the value planes of type T and their distance in elements
+template <class T> __device__ __forceinline__ const T* star_planes(const StarOpArgs& a);
+template <> __device__ __forceinline__ const double* star_planes<double>(const StarOpArgs& a) { return a.vals; }
+template <> __device__ __forceinline__ const float* star_planes<float>(const StarOpArgs& a) { return a.vals32; }
+template <class T> __device__ __forceinline__ long star_stride(const StarOpArgs& a) { return sizeof(T) == 8 ? a.stride : a.stride32; }
+
 // one slot of a row: y_row += A(row, col) x(col); STAGED: values / column index / x window from the stage
-template <int NP, bool STAGED>
-__device__ __forceinline__ void slot_product(const StarOpArgs& a, bool ok, int s, const double* sv, const int* vb, const unsigned* sc,
-                                             int cbase, const double* sx, int wlo, unsigned wn, double* acc, double* dg) {
+template <int NP, bool STAGED, class T>
+__device__ __forceinline__ void slot_product(const StarOpArgs& a, bool ok, int s, const T* sv, const int* vb, const unsigned* sc,
+                                             int cbase, const double* sx, int wlo, unsigned wn, double* acc, T* dg) {
   constexpr int F = NP == 1 ? 1 : 3;
   const unsigned c = !ok ? 0u : ((STAGED ? sc[s - cbase] : a.col[s]) & STAR_VMASK);
   const unsigned cw = c - (unsigned)wlo; // (wraps for columns below the window)
@@ -106,29 +131,32 @@ __device__ __forceinline__ void slot_product(const StarOpArgs& a, bool ok, int s
 #pragma unroll
   for (int k = 0; k < F; k++) x[k] = !ok ? 0.0 : (in ? sx[F * cw + k] : a.x[(size_t)F * c + k]);
 #pragma unroll
-  for (int p = 0; p < NP; p++) v[p] = !ok ? 0.0 : (STAGED ? sv[vb[p] + s] : a.vals[(size_t)p * a.stride + s]);
+  for (int p = 0; p < NP; p++)
+    v[p] = !ok ? 0.0 : (double)(STAGED ? sv[vb[p] + s] : star_planes<T>(a)[(size_t)p * star_stride<T>(a) + s]);
   if (dg) {
 #pragma unroll
-    for (int p = 0; p < NP; p++) dg[p] = v[p];
+    for (int p = 0; p < NP; p++) dg[p] = (T)v[p]; // (exact: v[p] is a widened T)
   }
   if constexpr (NP == 1) acc[0] += v[0] * x[0];
   else block_mac<NP>(v, x, acc);
 }
 
-template <int NP, int EPI, int NDOT, int LPR>
-__global__ void __launch_bounds__(tma_threads(NP, EPI, NDOT, LPR), 1) k_star_op_tma(const StarOpArgs a, const int nstages) {
-  using L = TmaLayout<NP>;
+template <int NP, int EPI, int NDOT, int LPR, class T>
+__global__ void __launch_bounds__(tma_threads(NP, EPI, NDOT, LPR, tma_groups<T>(LPR)), 1) k_star_op_tma(const StarOpArgs a, const int nstages) {
+  static_assert(sizeof(T) == 8 || (NDOT == 0 && (EPI == EPI_RESIDUAL || EPI == EPI_JACOBI)), "float planes: multigrid residual / smoother only");
+  using L = TmaLayout<NP, T>;
   constexpr int F = L::F;
-  constexpr int TMA_NW = tma_nw(LPR);
+  constexpr int TMA_NW = tma_nw(LPR);   // consumer warps of a group (one tile)
+  constexpr int G = tma_groups<T>(LPR);
   constexpr int RW = 32 / LPR;          // rows per consumer warp and tile
   extern __shared__ __align__(128) unsigned char smem[];
   uint64_t* full = reinterpret_cast<uint64_t*>(smem);
-  uint64_t* empty = full + TMA_MAX_STAGES;
+  uint64_t* empty = full + L::MAX_STAGES;
   unsigned char* stages = smem + L::HEAD;
   double* ybuf = reinterpret_cast<double*>(stages + (size_t)nstages * L::STAGE);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int ntiles = (a.nv + TMA_TR - 1) / TMA_TR;
-  const int sp = (int)(a.stride & 1);
+  const int sp = sizeof(T) == 8 ? (int)(a.stride & 1) : 0; // (float planes: stride32 is a multiple of 4)
   if (threadIdx.x == 0) {
     for (int s = 0; s < nstages; s++) { mbar_init(&full[s], tma_producers(NP, EPI, NDOT)); mbar_init(&empty[s], TMA_NW); }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -138,7 +166,7 @@ __global__ void __launch_bounds__(tma_threads(NP, EPI, NDOT, LPR), 1) k_star_op_
 #pragma unroll
   for (int j = 0; j < (NDOT > 0 ? NDOT : 1); j++) dsum[j] = 0.0;
 
-  if (warp >= TMA_NW) {
+  if (warp >= G * TMA_NW) {
     // ---------------- producers: ONE WARP PER COPY STREAM (value plane p, column indices, row pointers, gather window,
     // right-hand side).  Issuing a bulk copy costs a chain of R2UR / ELECT / UBLKCP instructions in a single thread; one
     // thread issuing all eleven copies of a tile needed ~4 300 cycles per tile and paced the whole kernel at 4.1 TB/s
@@ -147,7 +175,7 @@ __global__ void __launch_bounds__(tma_threads(NP, EPI, NDOT, LPR), 1) k_star_op_
     // The slot range of a tile comes from two row pointers in global memory; a load issued while the bulk copies
     // saturate DRAM takes microseconds, so every lane fetches the boundaries of one of the next 32 tiles, a full batch
     // ahead of their use, and lane 0 picks them up by shuffle.
-    const int role = warp - TMA_NW; // 0..NP-1: plane, NP: columns, NP+1: row pointers, NP+2: x window, NP+3: b / w1
+    const int role = warp - G * TMA_NW; // 0..NP-1: plane, NP: columns, NP+1: row pointers, NP+2: x window, NP+3: b / w1
     auto load_batch = [&](int batch, int& lo, int& hi) {
       const long tt = blockIdx.x + (long)(batch * 32 + lane) * gridDim.x;
       lo = 0; hi = 0;
@@ -167,46 +195,54 @@ __global__ void __launch_bounds__(tma_threads(NP, EPI, NDOT, LPR), 1) k_star_op_
         unsigned char* st = stages + (size_t)stage * L::STAGE;
         const int r0 = t * TMA_TR, rows = min(TMA_TR, a.nv - r0);
         const bool staged = hi - lo <= TMA_CAP;
-        const void* src = nullptr; void* dst = nullptr; unsigned nb = 0;
-        if (role < NP) {
-          if (staged) {
-            const int o = (lo + role * sp) & 1;
-            nb = (unsigned)(((hi - lo + o) + 1) & ~1) * 8u;
-            src = a.vals + (size_t)role * a.stride + (lo - o); dst = st + role * L::PLANE;
+        for (int k = 0; k < (tma_shared_rp_b(NP, EPI, NDOT, G) && role == NP + 1 ? 2 : 1); k++) {
+          const int rl = k == 0 ? role : NP + 3;
+          const void* src = nullptr; void* dst = nullptr; unsigned nb = 0;
+          if (rl < NP) {
+            if (staged && sizeof(T) == 8) {
+              const int o = (lo + rl * sp) & 1;
+              nb = (unsigned)(((hi - lo + o) + 1) & ~1) * 8u;
+              src = a.vals + (size_t)rl * a.stride + (lo - o); dst = st + rl * L::PLANE;
+            } else if (staged) { // float planes: the source rounded down to 4 slots, as the column stream
+              const int lo_v = lo & ~3;
+              nb = (unsigned)(((hi - lo_v) + 3) & ~3) * 4u;
+              src = a.vals32 + (size_t)rl * a.stride32 + lo_v; dst = st + rl * L::PLANE;
+            }
+          } else if (rl == NP) {
+            if (staged) {
+              const int lo_c = lo & ~3;
+              nb = (unsigned)(((hi - lo_c) + 3) & ~3) * 4u;
+              src = a.col + lo_c; dst = st + L::COLS;
+            }
+          } else if (rl == NP + 1) {
+            nb = (unsigned)((rows + 1 + 3) & ~3) * 4u;
+            src = a.rp + r0; dst = st + L::RP;
+          } else if (rl == NP + 2) {
+            const int wlo = max(r0 - TMA_W, 0), whi = min(r0 + TMA_TR + TMA_W, a.nv);
+            nb = (unsigned)((F * (whi - wlo) + 1) & ~1) * 8u;
+            src = a.x + (size_t)F * wlo; dst = st + L::XW;
+          } else {
+            nb = (unsigned)((F * rows + 1) & ~1) * 8u;
+            src = (EPI == EPI_PLAIN ? a.w1 : a.b) + (size_t)F * r0; dst = st + L::B;
           }
-        } else if (role == NP) {
-          if (staged) {
-            const int lo_c = lo & ~3;
-            nb = (unsigned)(((hi - lo_c) + 3) & ~3) * 4u;
-            src = a.col + lo_c; dst = st + L::COLS;
-          }
-        } else if (role == NP + 1) {
-          nb = (unsigned)((rows + 1 + 3) & ~3) * 4u;
-          src = a.rp + r0; dst = st + L::RP;
-        } else if (role == NP + 2) {
-          const int wlo = max(r0 - TMA_W, 0), whi = min(r0 + TMA_TR + TMA_W, a.nv);
-          nb = (unsigned)((F * (whi - wlo) + 1) & ~1) * 8u;
-          src = a.x + (size_t)F * wlo; dst = st + L::XW;
-        } else {
-          nb = (unsigned)((F * rows + 1) & ~1) * 8u;
-          src = (EPI == EPI_PLAIN ? a.w1 : a.b) + (size_t)F * r0; dst = st + L::B;
+          if (nb) { mbar_expect_tx(&full[stage], nb); bulk_g2s(dst, src, nb, &full[stage]); }
+          else mbar_arrive(&full[stage]);
         }
-        if (nb) { mbar_expect_tx(&full[stage], nb); bulk_g2s(dst, src, nb, &full[stage]); }
-        else mbar_arrive(&full[stage]);
       }
       __syncwarp();
     }
   } else {
-    // ---------------- consumers: lane <-> row (LPR lanes per row) ----------------
+    // ---------------- consumers: lane <-> row (LPR lanes per row); group `grp` takes tiles it = grp, grp + G, ... ----------------
     const int sub = lane % LPR;
+    const int grp = warp / TMA_NW, cwarp = warp % TMA_NW;
     double* yw = ybuf + warp * RW * F;
-    int t = blockIdx.x;
-    for (int it = 0; t < ntiles; t += gridDim.x, it++) {
+    int t = blockIdx.x + grp * gridDim.x;
+    for (int it = grp; t < ntiles; t += G * gridDim.x, it += G) {
       const int stage = it % nstages;
       const unsigned parity = (unsigned)((it / nstages) & 1);
       mbar_wait(&full[stage], parity);
       const unsigned char* st = stages + (size_t)stage * L::STAGE;
-      const double* sv = reinterpret_cast<const double*>(st);
+      const T* sv = reinterpret_cast<const T*>(st);
       const unsigned* sc = reinterpret_cast<const unsigned*>(st + L::COLS);
       const int* srp = reinterpret_cast<const int*>(st + L::RP);
       const double* sb = reinterpret_cast<const double*>(st + L::B);
@@ -220,15 +256,16 @@ __global__ void __launch_bounds__(tma_threads(NP, EPI, NDOT, LPR), 1) k_star_op_
       const int cbase = lo & ~3;
       int vb[NP]; // plane p, slot s -> sv[vb[p] + s]
 #pragma unroll
-      for (int p = 0; p < NP; p++) vb[p] = p * (TMA_CAP + 2) - lo + ((lo + p * sp) & 1);
-      const int rl = RW * warp + lane / LPR; // row of this lane inside the tile
+      for (int p = 0; p < NP; p++) vb[p] = sizeof(T) == 8 ? p * L::PSLOTS - lo + ((lo + p * sp) & 1) : p * L::PSLOTS - cbase;
+      const int rl = RW * cwarp + lane / LPR; // row of this lane inside the tile
       const bool valid = rl < rows;
       const int b0 = valid ? srp[rl] : hi, e0 = valid ? srp[rl + 1] : hi;
-      double acc[F], dg[NP];
+      double acc[F];
+      T dg[NP]; // the diagonal slot's values, kept in the plane type (fewer registers for float planes)
 #pragma unroll
       for (int k = 0; k < F; k++) acc[k] = 0.0;
 #pragma unroll
-      for (int p = 0; p < NP; p++) dg[p] = 0.0;
+      for (int p = 0; p < NP; p++) dg[p] = 0;
       const int len = e0 - b0;
       const int maxlen = __reduce_max_sync(0xffffffffu, len);
       if (staged) {
@@ -266,20 +303,20 @@ __global__ void __launch_bounds__(tma_threads(NP, EPI, NDOT, LPR), 1) k_star_op_
           const int s = b0 + sub + u * LPR;
           double v[NP];
 #pragma unroll
-          for (int p = 0; p < NP; p++) v[p] = okj[u] ? sv[vb[p] + s] : 0.0;
+          for (int p = 0; p < NP; p++) v[p] = okj[u] ? (double)sv[vb[p] + s] : 0.0;
           if (EPI == EPI_JACOBI && u == 0) {
 #pragma unroll
-            for (int p = 0; p < NP; p++) dg[p] = v[p];
+            for (int p = 0; p < NP; p++) dg[p] = (T)v[p];
           }
           if constexpr (NP == 1) acc[0] += v[0] * xj[u][0];
           else block_mac<NP>(v, xj[u], acc);
         }
         for (int j = sub + MAXS * LPR; j < maxlen; j += LPR) // rows with more slots (valence > 7)
-          slot_product<NP, true>(a, j < len, b0 + j, sv, vb, sc, cbase, sx, wlo, wn, acc, nullptr);
+          slot_product<NP, true, T>(a, j < len, b0 + j, sv, vb, sc, cbase, sx, wlo, wn, acc, nullptr);
       } else { // over-full tile: slots straight from global memory
-        slot_product<NP, false>(a, sub < len, b0 + sub, sv, vb, sc, cbase, sx, wlo, wn, acc, EPI == EPI_JACOBI ? dg : nullptr);
+        slot_product<NP, false, T>(a, sub < len, b0 + sub, sv, vb, sc, cbase, sx, wlo, wn, acc, EPI == EPI_JACOBI ? dg : nullptr);
         for (int j = sub + LPR; j < maxlen; j += LPR)
-          slot_product<NP, false>(a, j < len, b0 + j, sv, vb, sc, cbase, sx, wlo, wn, acc, nullptr);
+          slot_product<NP, false, T>(a, j < len, b0 + j, sv, vb, sc, cbase, sx, wlo, wn, acc, nullptr);
       }
       if (LPR > 1) {
 #pragma unroll
@@ -303,17 +340,19 @@ __global__ void __launch_bounds__(tma_threads(NP, EPI, NDOT, LPR), 1) k_star_op_
 #pragma unroll
           for (int k = 0; k < F; k++) yv[k] = sb[F * rl + k] - acc[k];
         } else { // damped (point-block) Jacobi step: y = x + omega * D^-1 (b - A x)
-          double r[F], z[F];
+          double r[F], z[F], dgd[NP];
+#pragma unroll
+          for (int p = 0; p < NP; p++) dgd[p] = dg[p];
 #pragma unroll
           for (int k = 0; k < F; k++) r[k] = sb[F * rl + k] - acc[k];
           if constexpr (F == 3) {
 #pragma unroll
             for (int k = 0; k < F; k++) {
               double o[3];
-              block_inverse_row<NP>(dg, k, o);
+              block_inverse_row<NP>(dgd, k, o);
               z[k] = o[0] * r[0] + o[1] * r[1] + o[2] * r[2];
             }
-          } else z[0] = (dg[0] != 0.0 ? 1.0 / dg[0] : 0.0) * r[0];
+          } else z[0] = (dgd[0] != 0.0 ? 1.0 / dgd[0] : 0.0) * r[0];
 #pragma unroll
           for (int k = 0; k < F; k++) yv[k] = sxo[F * rl + k] + a.omega * z[k];
         }
@@ -325,7 +364,7 @@ __global__ void __launch_bounds__(tma_threads(NP, EPI, NDOT, LPR), 1) k_star_op_
       __syncwarp();
       // this warp's RW*F results are contiguous in y
       {
-        const size_t g0 = (size_t)F * (r0 + RW * warp);
+        const size_t g0 = (size_t)F * (r0 + RW * cwarp);
         const size_t gend = (size_t)F * a.nv;
 #pragma unroll
         for (int i = lane; i < RW * F; i += 32)
@@ -336,19 +375,19 @@ __global__ void __launch_bounds__(tma_threads(NP, EPI, NDOT, LPR), 1) k_star_op_
     }
   }
   if (NDOT > 0) {
-    __shared__ double sm[NDOT > 0 ? NDOT : 1][TMA_NW];
+    __shared__ double sm[NDOT > 0 ? NDOT : 1][G * TMA_NW];
 #pragma unroll
     for (int j = 0; j < (NDOT > 0 ? NDOT : 1); j++) {
       double s = dsum[j];
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-      if (lane == 0 && warp < TMA_NW) sm[j][warp] = s;
+      if (lane == 0 && warp < G * TMA_NW) sm[j][warp] = s;
     }
     __syncthreads();
     if (warp == 0) {
 #pragma unroll
       for (int j = 0; j < (NDOT > 0 ? NDOT : 1); j++) {
-        double s = lane < TMA_NW ? sm[j][lane] : 0.0;
+        double s = lane < G * TMA_NW ? sm[j][lane] : 0.0;
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
         if (lane == 0) a.partial[(long)blockIdx.x * NDOT + j] = s;
@@ -364,7 +403,8 @@ inline bool star_op_tma_ok(const Ctx& c, const StarOpArgs& a, int epi) {
   if (!t.tma || epi == EPI_CHEBYSHEV) return false;
   if ((long)a.nv < (t.tma_min_rows >= 0 ? t.tma_min_rows : 2l * TMA_TR * c.sm_count)) return false;
   auto al = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
-  return al(a.rp) && al(a.col) && al(a.vals) && al(a.x) && (!a.b || al(a.b)) && (!a.w1 || al(a.w1));
+  return al(a.rp) && al(a.col) && al(a.vals) && (!a.vals32 || (al(a.vals32) && a.stride32 % 4 == 0)) && al(a.x) &&
+         (!a.b || al(a.b)) && (!a.w1 || al(a.w1));
 }
 
 inline int star_op_tma_stages() {
@@ -372,34 +412,41 @@ inline int star_op_tma_stages() {
   return v < 2 ? 2 : (v > TMA_MAX_STAGES ? TMA_MAX_STAGES : v);
 }
 
-template <int NP, int EPI, int NDOT, int LPR>
+template <int NP, int EPI, int NDOT, int LPR, class T>
 inline int launch_star_op_tma_lpr(Ctx& c, const StarOpArgs& a) {
-  using L = TmaLayout<NP>;
-  const int nstages = star_op_tma_stages();
+  using L = TmaLayout<NP, T>;
+  const int nstages = sizeof(T) == 8 ? star_op_tma_stages() : TMA_F32_STAGES;
   const int smem = L::smem_bytes(nstages);
   static unsigned long long configured = 0; // per device bit: the attribute is per device and function
   if (!(configured >> (c.device & 63) & 1ull)) {
-    PNP_CUDA(cudaFuncSetAttribute(k_star_op_tma<NP, EPI, NDOT, LPR>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::smem_bytes(TMA_MAX_STAGES)));
+    PNP_CUDA(cudaFuncSetAttribute(k_star_op_tma<NP, EPI, NDOT, LPR, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::smem_bytes(L::MAX_STAGES)));
     configured |= 1ull << (c.device & 63);
   }
   const int ntiles = (a.nv + TMA_TR - 1) / TMA_TR;
   const int grid = ntiles < c.sm_count ? ntiles : c.sm_count;
-  k_star_op_tma<NP, EPI, NDOT, LPR><<<grid, tma_threads(NP, EPI, NDOT, LPR), smem, c.stream>>>(a, nstages);
+  k_star_op_tma<NP, EPI, NDOT, LPR, T><<<grid, tma_threads(NP, EPI, NDOT, LPR, tma_groups<T>(LPR)), smem, c.stream>>>(a, nstages);
   PNP_CHECK_LAUNCH(); c.launches++;
   return grid;
 }
-template <int NP, int EPI, int NDOT>
+template <int NP, int EPI, int NDOT, class T>
 inline int launch_star_op_tma_inst(Ctx& c, const StarOpArgs& a) {
-  return tune().tma_lpr == 2 ? launch_star_op_tma_lpr<NP, EPI, NDOT, 2>(c, a) : launch_star_op_tma_lpr<NP, EPI, NDOT, 1>(c, a);
+  return tune().tma_lpr == 2 ? launch_star_op_tma_lpr<NP, EPI, NDOT, 2, T>(c, a) : launch_star_op_tma_lpr<NP, EPI, NDOT, 1, T>(c, a);
+}
+template <int EPI, int NDOT, class T>
+inline int launch_star_op_tma_planes(Ctx& c, int nplanes, const StarOpArgs& a) {
+  return nplanes == 1 ? launch_star_op_tma_inst<1, EPI, NDOT, T>(c, a)
+       : nplanes == PNP_COMPACT_PLANES ? launch_star_op_tma_inst<PNP_COMPACT_PLANES, EPI, NDOT, T>(c, a)
+                                       : launch_star_op_tma_inst<7, EPI, NDOT, T>(c, a);
 }
 
 // launches the streaming or the plain-load kernel; returns the grid size (number of partial-sum blocks)
-// compulsory traffic of one star-op launch: NP value planes + column index per slot; row pointer, x read once and y
-// written per row; the epilogue's extra vectors (b; the dot operand; the Chebyshev direction read and written)
+// compulsory traffic of one star-op launch: NP value planes (doubles, or the floats of vals32) + column index per slot;
+// row pointer, x read once and y written per row; the epilogue's extra vectors (b; the dot operand; the Chebyshev
+// direction read and written)
 template <int EPI, int NDOT>
 inline double star_op_bytes(int nplanes, const StarOpArgs& a) {
-  const double F = nplanes == 1 ? 1 : 3, nv = a.nv, ns = a.rp ? (double)a.stride : 0.0;
-  double b = (8.0 * nplanes + 4.0) * ns + (4.0 + 16.0 * F) * nv;
+  const double F = nplanes == 1 ? 1 : 3, nv = a.nv, ns = a.rp ? (double)a.stride : 0.0, vs = a.vals32 ? 4.0 : 8.0;
+  double b = (vs * nplanes + 4.0) * ns + (4.0 + 16.0 * F) * nv;
   if (EPI != EPI_PLAIN) b += 8.0 * F * nv;
   if (EPI == EPI_PLAIN && NDOT >= 1) b += 8.0 * F * nv;
   if (EPI == EPI_CHEBYSHEV) b += 16.0 * F * nv;
@@ -408,11 +455,17 @@ inline double star_op_bytes(int nplanes, const StarOpArgs& a) {
 template <int EPI, int NDOT>
 inline int launch_star_op_auto(Ctx& c, int nplanes, const StarOpArgs& a, bool fine = true) {
   c.acct(fine ? Ctx::ACC_SPMV_FINE : Ctx::ACC_SPMV_COARSE, star_op_bytes<EPI, NDOT>(nplanes, a));
-  if (EPI != EPI_CHEBYSHEV && star_op_tma_ok(c, a, EPI)) {
+  const bool tma = EPI != EPI_CHEBYSHEV && star_op_tma_ok(c, a, EPI);
+  if constexpr ((EPI == EPI_RESIDUAL || EPI == EPI_JACOBI) && NDOT == 0) {
+    if (a.vals32) {
+      PNP_REQUIRE(tma, PNP_E_ARG, "float value planes are read by the streaming SpMV only (a tma knob changed since the multigrid set-up)");
+      return launch_star_op_tma_planes<EPI, NDOT, float>(c, nplanes, a);
+    }
+  }
+  PNP_REQUIRE(!a.vals32, PNP_E_ARG, "float value planes: multigrid residual and smoother steps only");
+  if (tma) {
     constexpr int E = EPI == EPI_CHEBYSHEV ? EPI_PLAIN : EPI; // (never instantiated for Chebyshev)
-    return nplanes == 1 ? launch_star_op_tma_inst<1, E, NDOT>(c, a)
-         : nplanes == PNP_COMPACT_PLANES ? launch_star_op_tma_inst<PNP_COMPACT_PLANES, E, NDOT>(c, a)
-                                         : launch_star_op_tma_inst<7, E, NDOT>(c, a);
+    return launch_star_op_tma_planes<E, NDOT, double>(c, nplanes, a);
   }
   return launch_star_op<EPI, NDOT>(c, nplanes, a);
 }
